@@ -118,6 +118,25 @@ class ClockSampler:
                 "reasons": reasons, "samples": len(sm)}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each output of the last timed step as out_dir/<name>.npy: float64 stays float64, everything else
+    (float32 tracks, integer counts and indices, boolean masks) becomes float32.  At the C3 size the whole set is a
+    few MB, far under DUMP_LIMIT_BYTES, so every array is written in full."""
+    host = {}
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if hasattr(a, "detach") else np.asarray(a)
+        host[name] = a if a.dtype == np.float64 else a.astype(np.float32)
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def make_problem():
     from vggsfm_b200.synthetic import make_scene, perturb
     sc = make_scene(S_FRAMES, N_TRACKS, CAMERA, seed=0)
@@ -149,23 +168,10 @@ def cpu_ba_sample(sc, extr, K, extra, pts, iters):
 
 def cpu_tri_sample(sc, ntracks):
     """CPU triangulate_tracks (256 hypotheses) on the first `ntracks` tracks of C3; returns (tracks/s, seconds, kind).
-    kind = "reference": the reference's own triangulate_tracks (vggsfm/utils/triangulation.py:677) imported from
-    /root/reference with stub third-party modules (build container only -- the path does not exist on the GPU box);
     kind = "port": oracle/tri_oracle.py (numpy restatement pinned to the reference's goldens)."""
     import torch
-    from oracle import reference_shim, tri_oracle as to
+    from oracle import tri_oracle as to
     tn = to.cam_from_img(sc.tracks[:, :ntracks].astype(np.float64), sc.intrinsics, sc.extra_params)
-    if reference_shim.available():
-        reference_shim.install()
-        from vggsfm.utils.triangulation import triangulate_tracks as ref_tt
-        torch.set_num_threads(os.cpu_count() or 1)
-        E = torch.from_numpy(sc.extrinsics)
-        tnt = reference_shim.contiguous_tracks(torch.from_numpy(tn))
-        torch.manual_seed(0)
-        t0 = time.perf_counter()
-        ref_tt(E, tnt, track_vis=torch.from_numpy(sc.vis[:, :ntracks]), track_score=torch.from_numpy(sc.score[:, :ntracks]))
-        dt = time.perf_counter() - t0
-        return ntracks / dt, dt, "reference"
     torch.manual_seed(0)
     pairs = to.draw_pairs(S_FRAMES, 256)
     t0 = time.perf_counter()
@@ -445,7 +451,8 @@ def run_gpu(args):
 
     def ba_step():
         poses, intr, X = poses0.clone(), intr0.clone(), pts0.clone()
-        return ba.lm_solve(uv, mask, poses, intr, X, model, mode, param_const, None, opt, hook)
+        s = ba.lm_solve(uv, mask, poses, intr, X, model, mode, param_const, None, opt, hook)
+        return s, {"ba_poses": poses, "ba_intrinsics": intr, "ba_points3d": X}
 
     # ---- timed region 1: BA
     launches = 0
@@ -463,7 +470,7 @@ def run_gpu(args):
     its = 0
     for _ in range(args.steps):
         flush.fill_(1.0)
-        s = ba_step()
+        s, ba_out = ba_step()
         its += s.iterations
         launches += s.kernel_launches
     e1.record()
@@ -498,7 +505,7 @@ def run_gpu(args):
     e0.record()
     for _ in range(args.steps):
         flush.fill_(1.0)
-        p3, num, _ = tri_pass()
+        p3, num, inl = tri_pass()
         launches += 6
     e1.record()
     barrier()
@@ -524,7 +531,7 @@ def run_gpu(args):
                                    h_tracks.to(dev, non_blocking=True), h_masks.to(dev, non_blocking=True),
                                    shared_camera=True, camera_type=CAMERA, options=opt, allreduce=hook)
         res = [out[0].cpu(), out[1].cpu(), out[2].cpu(), out[3].cpu()]
-        return out[5], sum(x.numel() * x.element_size() for x in res)
+        return out[5], sum(x.numel() * x.element_size() for x in res), res + [out[4]]
 
     for _ in range(min(args.warmup, 2)):
         e2e_step()
@@ -533,7 +540,7 @@ def run_gpu(args):
     e2e_its = 0
     d2h = 0
     for _ in range(args.steps):
-        s2, d2h = e2e_step()
+        s2, d2h, e2e_out = e2e_step()
         e2e_its += s2.iterations
         launches += s2.kernel_launches
     barrier()
@@ -542,6 +549,11 @@ def run_gpu(args):
     if world > 1:
         dist.all_reduce(ts, op=dist.ReduceOp.MAX)
     e2e_value = e2e_its / float(ts.item())
+
+    if rank == 0 and args.dump_outputs:
+        names = ("e2e_points3d", "e2e_extrinsics", "e2e_intrinsics", "e2e_extra_params", "e2e_valid_idx")
+        dump_outputs(args.dump_outputs, {**ba_out, "tri_points3d": p3, "tri_inlier_num": num, "tri_inlier_mask": inl,
+                                         **dict(zip(names, e2e_out))})
 
     # ---- roofline of the fused residual+Jacobian+block kernel (the HBM-bound kernel of the path), live
     roof = None
@@ -688,7 +700,14 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-corr", action="store_true", help="skip the C4 correlation section (rank 0, N=1 only)")
     ap.add_argument("--no-c5", action="store_true", help="skip the C5 sequential-video section (rank 0, N=1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last BA, triangulation and end-to-end steps returned as "
+                         "DIR/<name>.npy (float32/float64; rank 0's shard of the tracks when N>1)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,19 +1,19 @@
-"""Import the UNMODIFIED reference (/root/reference) with stub third-party modules -- TEST INFRASTRUCTURE ONLY.
+"""Import the UNMODIFIED reference (facebookresearch/vggsfm) with stub third-party modules -- TEST INFRASTRUCTURE ONLY.
 
-Used in the build container (where /root/reference exists) to validate the oracle restatements and to
-generate the golden fixtures under tests/golden/ (tools/make_golden.py).  /root/reference does not exist
-on the GPU box: nothing in the `-m gpu` tests, smoke() or bench.py calls this module.
+Used by the golden generators under tools/ to produce the fixtures in tests/golden/ from a checkout of the reference
+named by the VGGSFM_REFERENCE environment variable.  The test suite, smoke() and bench.py never call this module: they
+compare against the stored fixtures.
 Recipe: SURVEY.md Appendix C.
 """
 import os
 import sys
 import types
 
-REFERENCE_ROOT = "/root/reference"
+REFERENCE_ROOT = os.environ.get("VGGSFM_REFERENCE", "")
 
 
 def available() -> bool:
-    return os.path.isdir(os.path.join(REFERENCE_ROOT, "vggsfm"))
+    return bool(REFERENCE_ROOT) and os.path.isdir(os.path.join(REFERENCE_ROOT, "vggsfm"))
 
 
 class _Stub(types.ModuleType):
@@ -38,7 +38,7 @@ _STUBS = ["hydra", "hydra.utils", "pycolmap", "pyceres", "kornia", "kornia.core"
 def install():
     """Put the reference on sys.path with stubs for the absent third-party packages."""
     if not available():
-        raise RuntimeError("/root/reference is not present on this machine")
+        raise RuntimeError("set VGGSFM_REFERENCE to a checkout of facebookresearch/vggsfm")
     import torch
     for name in _STUBS:
         sys.modules.setdefault(name, _Stub(name))

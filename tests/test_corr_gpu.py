@@ -18,7 +18,8 @@ GOLDEN = sorted(glob.glob(os.path.join(os.path.dirname(__file__), "golden", "cor
 def test_against_reference_golden(cuda_dev, path):
     from vggsfm_b200.corr import CorrBlock, EfficientCorrBlock
     g = np.load(path)
-    f, t, c = (torch.from_numpy(g[k]).to(cuda_dev) for k in ("fmaps", "targets", "coords"))
+    # fmaps are stored as float16, exactly the values the reference ran on
+    f, t, c = (torch.from_numpy(g[k].astype(np.float32)).to(cuda_dev) for k in ("fmaps", "targets", "coords"))
     L, r = int(g["num_levels"]), int(g["radius"])
     cb = CorrBlock(f, num_levels=L, radius=r, half=False)
     cb.corr(t)

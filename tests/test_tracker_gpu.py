@@ -37,7 +37,8 @@ def test_track_predictor_forward_matches_reference(cuda_dev):
     from vggsfm_b200 import tracker as tk
     g = np.load(os.path.join(GOLD, "tracker_coarse.npz"))
     p = _predictor(g, cuda_dev, 4, 5, 3, False, 1)
-    preds, vis, feats, qfeat = tk.track_predictor_forward(p, to_dev(g["qp"], cuda_dev), to_dev(g["fmaps"], cuda_dev), iters=4,
+    fmaps = to_dev(g["fmaps"].astype(np.float32), cuda_dev)            # stored as float16, exactly what the reference ran on
+    preds, vis, feats, qfeat = tk.track_predictor_forward(p, to_dev(g["qp"], cuda_dev), fmaps, iters=4,
                                                          return_feat=True)
     assert len(preds) == 4
     got = torch.stack(preds).cpu().numpy()

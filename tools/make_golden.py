@@ -1,7 +1,7 @@
-"""Generate tests/golden/*.npz by running the UNMODIFIED reference (/root/reference, imported with stub
-third-party modules) on seeded synthetic inputs.  Run in the build container only:
+"""Generate tests/golden/tri_*.npz and triangulate_tracks_10x40_radial.npz by running the UNMODIFIED reference
+(imported with stub third-party modules) on seeded synthetic inputs.  Needs a reference checkout:
 
-    python tools/make_golden.py
+    VGGSFM_REFERENCE=/path/to/vggsfm python tools/make_golden.py
 
 Pinned cases run the reference with torch.sort forced stable (its unstable descending sort leaves the
 order of equal inlier counts implementation-defined, see oracle/tri_oracle.py); the `unpinned` case runs
@@ -78,6 +78,20 @@ def main():
             filt_valid=v.numpy(), filt_detail=d.numpy(), filt_valid_notri=v2.numpy(), proj2d=p2d.numpy(),
             projcam=pcam.numpy(), pair_points=bp.numpy(), pair_cheirality=bche.numpy(), pair_angle=bang.numpy())
         print(name, "inliers/track mean", n.float().mean().item(), "valid", int(v.sum()))
+    # triangulate_tracks alone on a radial scene with outliers, stable sort, default arguments (256 hypotheses)
+    sc = make_scene(10, 40, "SIMPLE_RADIAL", seed=21, invisible_frac=0.2, outlier_frac=0.1)
+    tn = rh.cam_from_img(torch.from_numpy(sc.tracks), torch.from_numpy(sc.intrinsics), torch.from_numpy(sc.extra_params))
+    torch.manual_seed(3)
+    torch.sort = _stable_sort
+    try:
+        p, n, m = rt.triangulate_tracks(torch.from_numpy(sc.extrinsics), rs.contiguous_tracks(tn),
+                                        track_vis=torch.from_numpy(sc.vis), track_score=torch.from_numpy(sc.score))
+    finally:
+        torch.sort = _sort
+    np.savez_compressed(os.path.join(out_dir, "triangulate_tracks_10x40_radial.npz"), extrinsics=sc.extrinsics,
+                        tn=tn.numpy(), vis=sc.vis, score=sc.score, points=p.numpy(), inlier_num=n.numpy(),
+                        inlier_mask=m.numpy())
+    print("triangulate_tracks_10x40_radial", "inliers/track mean", n.float().mean().item())
 
 
 if __name__ == "__main__":

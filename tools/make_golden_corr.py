@@ -1,5 +1,6 @@
-"""Golden fixtures for the correlation path from the UNMODIFIED reference CorrBlock / EfficientCorrBlock
-(build container only):  python tools/make_golden_corr.py"""
+"""Golden fixtures for the correlation path from the UNMODIFIED reference CorrBlock / EfficientCorrBlock.  The feature
+maps are rounded to float16 before the run and stored as float16 (exact, and half the size).  Needs a reference
+checkout:  VGGSFM_REFERENCE=/path/to/vggsfm python tools/make_golden_corr.py"""
 import os
 import sys
 import warnings
@@ -26,7 +27,7 @@ def main():
     out_dir = os.path.join(ROOT, "tests", "golden")
     for name, (B, S, C, H, W, N, L, r, (lo, hi)) in CASES.items():
         g = torch.Generator().manual_seed(len(name))
-        fmaps = torch.randn(B, S, C, H, W, generator=g)
+        fmaps = torch.randn(B, S, C, H, W, generator=g).half().float()
         targets = torch.randn(B, S, N, C, generator=g)
         coords = torch.rand(B, S, N, 2, generator=g) * (hi - lo) + lo
         coords[0, 0, 0] = torch.tensor([3.0, 7.0])          # exactly integer coordinates
@@ -35,8 +36,7 @@ def main():
         out = cb.sample(coords)
         eb = EfficientCorrBlock(fmaps, num_levels=L, radius=r)
         out_b = eb.sample(coords, targets)
-        np.savez_compressed(os.path.join(out_dir, name + ".npz"), fmaps=fmaps.numpy().astype(np.float16).astype(np.float32)
-                            if False else fmaps.numpy(), targets=targets.numpy(), coords=coords.numpy(),
+        np.savez_compressed(os.path.join(out_dir, name + ".npz"), fmaps=fmaps.half().numpy(), targets=targets.numpy(), coords=coords.numpy(),
                             num_levels=L, radius=r, out_zeros=out.numpy(), out_border=out_b.numpy())
         print(name, out.shape, float(out.abs().mean()))
 

@@ -6,12 +6,15 @@ inverse ``pycolmap_to_batch_matrix`` (:163-214) with ``vggsfm_b200.reconstructio
 ``pycolmap`` module -- i.e. the reference's own O(S*P) Python loops decide ids, point2D order, the 3000 clamp and the
 camera sharing, and only the passive container classes are ours.  The flattened result is what
 ``Reconstruction.from_batch_matrix`` (the vectorised product path) must reproduce exactly.  Also pins the pure-torch
-``get_valid_frame_mask`` (vggsfm/utils/triangulation.py:1222-1242).  Needs /root/reference; run in the build container:
+``get_valid_frame_mask`` (vggsfm/utils/triangulation.py:1222-1242), and records how the reference's COLMAP reader
+(vggsfm/datasets/imc_helper.py:127-466) parses the binary model this package writes.  Needs a reference checkout:
 
-    python tools/make_golden_marshal.py
+    VGGSFM_REFERENCE=/path/to/vggsfm python tools/make_golden_marshal.py
 """
 import os
 import sys
+import tempfile
+import types
 
 import numpy as np
 import torch
@@ -61,6 +64,36 @@ def flatten(model):
     return o
 
 
+def read_back(path):
+    """The reference reader's view of the binary model under ``path`` -> flat arrays (the .bin bytes it parsed included)."""
+    sys.modules.setdefault("h5py", types.ModuleType("h5py"))          # imported at module scope there, unused by the readers
+    from vggsfm.datasets import imc_helper as ih
+    cams, ims, pts = ih.read_model(path, ext=".bin")
+    o = {}
+    for f in ("cameras", "images", "points3D"):
+        with open(os.path.join(path, f + ".bin"), "rb") as fh:
+            o["bin_" + f] = np.frombuffer(fh.read(), dtype=np.uint8)
+    cids, iids, pids = sorted(cams), sorted(ims), sorted(pts)
+    o["cam_ids"] = np.array(cids)
+    o["cam_model"] = np.array([cams[c].model for c in cids])
+    o["cam_wh"] = np.array([[cams[c].width, cams[c].height] for c in cids])
+    o["cam_params"] = np.stack([cams[c].params for c in cids])
+    o["img_ids"] = np.array(iids)
+    o["img_name"] = np.array([ims[i].name for i in iids])
+    o["img_cam"] = np.array([ims[i].camera_id for i in iids])
+    o["img_R"] = np.stack([ims[i].qvec2rotmat() for i in iids])
+    o["img_tvec"] = np.stack([ims[i].tvec for i in iids])
+    o["img_npts"] = np.array([len(ims[i].point3D_ids) for i in iids])
+    o["img_xys"] = np.concatenate([ims[i].xys.reshape(-1, 2) for i in iids])
+    o["img_p3d"] = np.concatenate([ims[i].point3D_ids.reshape(-1) for i in iids])
+    o["pt_ids"] = np.array(pids)
+    o["pt_xyz"] = np.stack([pts[p].xyz for p in pids])
+    o["pt_rgb"] = np.stack([pts[p].rgb for p in pids])
+    o["pt_tracklen"] = np.array([len(pts[p].image_ids) for p in pids])
+    o["pt_track"] = np.concatenate([np.stack([pts[p].image_ids, pts[p].point2D_idxs], 1).reshape(-1, 2) for p in pids])
+    return o
+
+
 def main():
     reference_shim.install()
     import vggsfm_b200.reconstruction as rc
@@ -96,6 +129,16 @@ def main():
     np.savez_compressed(os.path.join(ROOT, "tests", "golden", "valid_frame_mask.npz"), K=K.numpy(), E=E.numpy(), ex=ex.numpy(),
                         m1=m1.numpy(), m2=m2.numpy(), m3=m3.numpy())
     print("valid_frame_mask", m1.tolist())
+    # case c built by this package's vectorised path, written as COLMAP binaries, parsed by the reference's reader
+    c = cases()[2]
+    rec = rc.batch_matrix_to_pycolmap(t(c["pts"]), t(c["extr"]), t(c["K"]), t(c["tracks"]), t(c["masks"]), t(c["size"]),
+                                      shared_camera=c["shared"], camera_type=c["cam"], extra_params=t(c["extra"]))
+    rec.set_point_colors(np.linspace(0, 1, rec.num_points3D())[:, None].repeat(3, 1))
+    with tempfile.TemporaryDirectory() as d:
+        rec.write(d)
+        back = read_back(d)
+    np.savez_compressed(os.path.join(ROOT, "tests", "golden", "marshal_c_reader.npz"), **back)
+    print("marshal_c_reader", {k: v.shape for k, v in back.items()})
 
 
 if __name__ == "__main__":

@@ -5,7 +5,8 @@
 learned transformer is replaced on both sides by the deterministic stand-in tests/helpers.py:tiny_former (it is not on
 the hot path and its weights would not fit a fixture), the fine feature net by one 3x3 convolution.  kornia is absent:
 its two tiny functions used by compute_score_fn (create_meshgrid, dsnt.spatial_expectation2d) are restated here
-[3P-memory].  Needs /root/reference:   python tools/make_golden_tracker.py"""
+[3P-memory].  The coarse feature maps are rounded to float16 before the run and stored as float16 (exact, and half the
+size).  Needs a reference checkout:   VGGSFM_REFERENCE=/path/to/vggsfm python tools/make_golden_tracker.py"""
 import os
 import sys
 import types
@@ -35,6 +36,19 @@ def spatial_expectation2d(inp, normalized_coordinates=True):
     return torch.cat([ex, ey], dim=-1)
 
 
+def score_fn_inputs():
+    """(B, N, S, query features, patch features, tracks) of the compute_score_fn cases: C = 8, 31x31 patches, sradius 2;
+    some neighbourhoods get clamped at the patch border."""
+    g = torch.Generator().manual_seed(0)
+    out = []
+    for B, N, S in ((1, 5, 4), (2, 3, 3)):
+        qf = torch.randn(B, N, 8, generator=g)
+        pf = torch.randn(B * N, S, 8, 31, 31, generator=g)
+        trk = torch.rand(B * N, S, 1, 2, generator=g) * 34 - 2
+        out.append((B, N, S, qf, pf, trk))
+    return out
+
+
 def state(m):
     return {k: v.detach().numpy() for k, v in m.state_dict().items()}
 
@@ -57,10 +71,10 @@ def main():
         # smooth feature maps (a coarse random field, bilinearly upsampled, + 5 % noise): the correlation landscape a
         # trained encoder produces, not white noise
         fmaps = torch.nn.functional.interpolate(torch.randn(10, 32, 5, 7), size=(32, 48), mode="bilinear", align_corners=True)
-        fmaps = (fmaps + 0.05 * torch.randn_like(fmaps)).reshape(2, 5, 32, 32, 48)
+        fmaps = (fmaps + 0.05 * torch.randn_like(fmaps)).reshape(2, 5, 32, 32, 48).half().float()
         qp = torch.rand(2, 20, 2) * torch.tensor([48 * 4 - 8.0, 32 * 4 - 8.0]) + 4.0
         preds, vis, feats, qfeat = ref(qp, fmaps, iters=4, return_feat=True)
-        np.savez_compressed(os.path.join(out, "tracker_coarse.npz"), fmaps=fmaps.numpy(), qp=qp.numpy(),
+        np.savez_compressed(os.path.join(out, "tracker_coarse.npz"), fmaps=fmaps.half().numpy(), qp=qp.numpy(),
                             preds=torch.stack(preds).numpy(), vis=vis.numpy(), feats=feats.numpy(), qfeat=qfeat.numpy(),
                             transformer_dim=ref.transformer_dim,
                             **{"norm." + k: v for k, v in state(ref.norm).items()},
@@ -92,6 +106,13 @@ def main():
                             e64c=get_2d_embedding(xy, 64, cat_coords=True).numpy(),
                             pos216=get_2d_sincos_pos_embed(216, grid_size=(31, 31)).numpy(),
                             pos664=get_2d_sincos_pos_embed(664, grid_size=(6, 9)).numpy())
+        # ---- compute_score_fn, including the reference's two indexing quirks (refine_track.py:256-276), on the seeded
+        # inputs of score_fn_inputs(); the patch features are too large to store, a fixed sample of them pins the draw
+        rec = {}
+        for k, (B, N, S, qf, pf, trk) in enumerate(score_fn_inputs()):
+            rec[f"score{k}"] = rt.compute_score_fn(qf, pf, trk, 2, 31, B, N, S, 8).numpy()
+            rec[f"qf{k}"], rec[f"trk{k}"], rec[f"pf_sample{k}"] = qf.numpy(), trk.numpy(), pf.reshape(-1)[::97].numpy()
+        np.savez_compressed(os.path.join(out, "tracker_score_fn.npz"), **rec)
 
 
 if __name__ == "__main__":
