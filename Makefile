@@ -15,7 +15,7 @@ $(BUILD)/%.o: $(CSRC)/%.cu $(CSRC)/common.cuh include/vggsfm_b200.h
 	$(NVCC) $(NVFLAGS) -c $< -o $@ 2> $(BUILD)/$*.ptxas.log || (cat $(BUILD)/$*.ptxas.log; exit 1)
 
 $(LIB): $(OBJS)
-	$(NVCC) -shared $(ARCH) -o $@ $(OBJS) -L/usr/local/cuda/lib64 -lcusolver -lcublas -lcudart -Xlinker -rpath -Xlinker /usr/local/cuda/lib64
+	$(NVCC) -shared $(ARCH) -o $@ $(OBJS) -L/usr/local/cuda/lib64 -lcublas -lcudart -Xlinker -rpath -Xlinker /usr/local/cuda/lib64
 
 oracle:
 	$(MAKE) -C oracle

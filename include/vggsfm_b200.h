@@ -143,7 +143,7 @@ int vgg_cholesky_lower(int n, int lda, double* A, void* workspace, size_t ws_byt
 /* The same SYRK step on the tensor cores (csrc/syrk_i8.cu): Cmat[Dpad,Dpad] -= Zt^T Zt for Zt double [Kpad,Dpad]
  * (Dpad a multiple of 128), FP64-equivalent through `slices` (3..7; 7 = 54 fractional bits) int8
  * Ozaki slices on tcgen05.mma kind::i8 with exact int32 accumulation in TMEM.  The row-major LOWER triangle is written.
- * Selected inside vgg_ba_solve by VGG_SYRK=ozaki[:slices]; exposed for the parity tests and profiling. */
+ * vgg_ba_solve uses it with 7 slices; exposed for the parity tests and profiling. */
 int vgg_syrk_ozaki_workspace_bytes(int Kpad, int Dpad, int slices, size_t* bytes);
 int vgg_syrk_ozaki(int Kpad, int Dpad, const double* Zt, double* Cmat, int slices, void* workspace, size_t ws_bytes,
                    void* stream);

@@ -1,7 +1,7 @@
 """tcgen05 INT8 (Ozaki) SYRK (csrc/syrk_i8.cu, vgg_syrk_ozaki) against numpy float64: the error of every entry is
 bounded relative to (|Z|^T |Z|)_ij -- the quantity a float64 dot product's own rounding error is bounded by --
-at 2^-44 for 7 slices; fewer slices lose 8 bits each.  Also: the LM solve with VGG_SYRK=ozaki semantics is covered
-by tests/test_ba_gpu.py when that variable is set (tools/microbench.py ba A/B)."""
+at 2^-44 for 7 slices; fewer slices lose 8 bits each.  The LM solve, which runs this SYRK with 7 slices, is covered by
+tests/test_ba_gpu.py."""
 import ctypes
 
 import numpy as np
@@ -61,21 +61,6 @@ def test_accumulates_and_flags_nonfinite(cuda_dev):
     ok = np.ones(256, bool)
     ok[40] = False
     assert np.isfinite(got[np.ix_(ok, ok)]).all()
-
-
-def test_cta_pair_variant_in_subprocess(cuda_dev):
-    """VGG_SYRK_PAIR=1 (cta_group::2 cluster kernel; the switch is read once per process): same accuracy."""
-    import os
-    import re
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    env = dict(os.environ, VGG_SYRK_PAIR="1")
-    out = subprocess.run([sys.executable, os.path.join(root, "tools", "syrk_i8_check.py"), "384", "1024", "7"], env=env,
-                         capture_output=True, text=True, timeout=120)
-    assert out.returncode == 0, out.stderr[-500:]
-    m = re.search(r"= ([0-9.e+-]+)\s+symmetric", out.stdout)
-    assert m and float(m.group(1)) < 2.0 ** -44, out.stdout[-300:]
 
 
 def test_band_hint_skips_only_zero_blocks(cuda_dev):

@@ -1,4 +1,4 @@
-"""Accuracy / timing check of the tcgen05 INT8 (Ozaki) SYRK against numpy float64 and the DMMA kernel path.
+"""Accuracy / timing check of the tcgen05 INT8 (Ozaki) SYRK against numpy float64.
    python tools/syrk_i8_check.py [Dpad Kpad slices]"""
 import ctypes
 import os
@@ -12,13 +12,6 @@ sys.path.insert(0, ROOT)
 from vggsfm_b200 import _lib       # noqa: E402
 
 dev = torch.device("cuda:0")
-if len(sys.argv) > 1 and sys.argv[1] == "probe":
-    L = _lib.lib()
-    torch.zeros(1, device=dev)
-    o = (ctypes.c_int * 3)()
-    _lib.check(L.vgg_probe_remote_mbarrier(o, None), "probe")
-    print("remote-mbarrier probe: leader barrier completed =", o[0], " peer bytes landed =", o[1], " leader bytes landed =", o[2])
-    sys.exit(0)
 if len(sys.argv) > 1 and sys.argv[1] == "rate":
     L = _lib.lib()
     torch.zeros(1, device=dev)

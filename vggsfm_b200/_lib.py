@@ -26,7 +26,7 @@ EXPORTS = [
 
 
 # development probes (csrc/dev_probes.h): exported, not part of the public header
-DEV_EXPORTS = ["vgg_syrk_ozaki_mma_rate", "vgg_probe_remote_mbarrier", "vgg_dev_blocks_timing", "vgg_dev_blocks_last_ms",
+DEV_EXPORTS = ["vgg_syrk_ozaki_mma_rate", "vgg_dev_blocks_timing", "vgg_dev_blocks_last_ms",
                "vgg_dev_chol128_probe", "vgg_dev_set_syrk_ranges", "vgg_dev_trsv_probe", "vgg_dev_set_chol_band"]
 
 
@@ -141,10 +141,9 @@ def lib() -> ctypes.CDLL:
     L.vgg_absolute_pose_estimation.argtypes = [ci, ci, ci, vp, vp, vp, vp, vp, vp, ci, ci, cd, vp, vp, vp, vp, vp, cs, vp]
     L.vgg_syrk_ozaki_workspace_bytes.argtypes = [ci, ci, ci, ctypes.POINTER(cs)]
     L.vgg_syrk_ozaki_mma_rate.argtypes = [ci, ci, ctypes.POINTER(cd), vp]
-    L.vgg_probe_remote_mbarrier.argtypes = [ctypes.POINTER(ctypes.c_int), vp]
     L.vgg_dev_blocks_timing.argtypes = [ci]
     L.vgg_dev_blocks_last_ms.argtypes = [ctypes.POINTER(cd)]
-    L.vgg_dev_chol128_probe.argtypes = [ci, ci, vp, vp, vp]
+    L.vgg_dev_chol128_probe.argtypes = [ci, vp, vp, vp]
     L.vgg_dev_set_syrk_ranges.argtypes = [vp, ci]
     L.vgg_dev_trsv_probe.argtypes = [ci, ci, vp, vp, vp, vp]
     L.vgg_dev_set_chol_band.argtypes = [vp, ci, ci]

@@ -41,10 +41,9 @@ class _Pyramid:
                        "vgg_corr_build_pyramid")
         self.dev = dev
         # coarse tracker (C = 128, power-of-two maps, half pyramid): operand tile images for the tcgen05 kernel
-        # (csrc/corr_tc.cu); VGG_CORR_TC=0 keeps the CUDA-core footprint kernel for A/B
-        import os
+        # (csrc/corr_tc.cu); tc=False keeps the CUDA-core footprint kernel
         self.tc_tiles = None
-        want_tc = (os.environ.get("VGG_CORR_TC", "1") != "0") if tc is None else bool(tc)
+        want_tc = True if tc is None else bool(tc)
         if self.elem == 2 and want_tc and L.vgg_corr_tc_supported(C, H, W, num_levels, radius):
             tb = ctypes.c_size_t()
             _lib.check(L.vgg_corr_tc_bytes(B * S, C, H, W, num_levels, 0, ctypes.byref(tb), None), "vgg_corr_tc_bytes")

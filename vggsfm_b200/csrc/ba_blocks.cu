@@ -23,7 +23,6 @@
 //   * observations (uv 8 B + mask 1 B) are read with 32-byte vector loads, 4 tracks per lane at a time,
 //     prefetched one batch ahead; poses/intrinsics sit transposed in shared memory (one frame per lane).
 // Algorithmic HBM bytes per observation: 9 + 24*dc (+ amortised per-frame/per-point terms), see DESIGN.md.
-#include <stdlib.h>
 #include <utility>
 #include "common.cuh"
 #include "dev_probes.h"
@@ -390,7 +389,6 @@ static int launch_blocks(const vgg_ba_problem* p, double* cost, double* camrec, 
                       sizeof(float) * BW * 2 * 32 * 12;
   const bool tma_ok = ((reinterpret_cast<uintptr_t>(W) & 15) == 0);
   const int ngroups = (S + 31) / 32;
-  static const int minb = [] { const char* e = getenv("VGG_K1_MINB"); return (e && e[0] == '3') ? 3 : 2; }();
   if (tracks_per_warp <= 0 && g_band_dev.fg_tracks) {
     // banded (sequential) problems: most (frame group, track chunk) warps return at once, so the chunks must be small
     // enough for the few that do not to spread over the machine (r02 launch list at 1000 frames x 32 k points: with the
@@ -401,18 +399,15 @@ static int launch_blocks(const vgg_ba_problem* p, double* cost, double* camrec, 
     // Every warp does the same amount of work, so the grid must be a whole number of waves: resident warps =
     // SMs x CTAs/SM (occupancy query) x BW.  Pick the smallest wave count that keeps >= 32 tracks per warp
     // amortising the per-warp camera flush (32 x KR REDs), capped at 4 waves; tracks per warp multiple of TB.
-    static int slots_cache[2] = {0, 0};
-    int& slots = slots_cache[minb == 3];
+    static int slots = 0;
     if (slots == 0) {
-      int dev = 0, sms = 148, per_sm = minb;
+      int dev = 0, sms = 148, per_sm = 2;
       cudaGetDevice(&dev);
       cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
       // the occupancy query needs the opt-in shared-memory limit in place (r02: without it the query returned 0, the
       // grid was sized for ONE CTA per SM and the 400 x 4096 launch ran as a single wave of 147 CTAs, half the warps)
       cudaFuncSetAttribute(ba_blocks_kernel<MODEL, MODE, true, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      cudaFuncSetAttribute(ba_blocks_kernel<MODEL, MODE, true, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      if (minb == 3) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ba_blocks_kernel<MODEL, MODE, true, 3>, BT, smem);
-      else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ba_blocks_kernel<MODEL, MODE, true, 2>, BT, smem);
+      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ba_blocks_kernel<MODEL, MODE, true, 2>, BT, smem);
       if (per_sm < 1) per_sm = 1;
       slots = sms * per_sm;
     }
@@ -455,16 +450,11 @@ static int launch_blocks(const vgg_ba_problem* p, double* cost, double* camrec, 
     const size_t tail = pitch - (size_t)S * C::DC;
     VGG_CUDA_CHECK(cudaMemset2DAsync(W + (size_t)S * C::DC * 3, pitch * 24, 0, tail * 24, (size_t)N, stream));
   }
-  // MINB = 3 caps registers at 168 (12 resident warps/SM, a few spills); MINB = 2 lets ptxas use ~250 (no spills,
-  // 8 warps/SM) and is the default.  VGG_K1_MINB=2|3 selects for A/B runs.
+  // Aligned W: MINB = 2 lets ptxas use ~250 registers (no spills, 8 warps/SM).  Unaligned W (no bulk copies) keeps the
+  // MINB = 3 build (168 registers, 12 warps/SM, a few spills).
   if (g_blocks_timing) VGG_CUDA_CHECK(cudaEventRecord(g_blocks_ev[0], stream));
-  if (tma_ok && minb == 2) {
+  if (tma_ok) {
     auto kern = ba_blocks_kernel<MODEL, MODE, true, 2>;
-    VGG_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid, BT, smem, stream>>>(S, N, tracks_per_warp, p->uv, p->mask, p->poses, p->intr, p->points,
-                                     p->point_const, cost, camrec, g_p, H_pp, W, shared_out, g_band_dev.fg_tracks);
-  } else if (tma_ok) {
-    auto kern = ba_blocks_kernel<MODEL, MODE, true, 3>;
     VGG_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kern<<<grid, BT, smem, stream>>>(S, N, tracks_per_warp, p->uv, p->mask, p->poses, p->intr, p->points,
                                      p->point_const, cost, camrec, g_p, H_pp, W, shared_out, g_band_dev.fg_tracks);

@@ -8,12 +8,10 @@
 //   assemble_hc     camera Hessian/gradient from the per-frame records into the dense reduced system
 //   z_build         Zt[3n+c][row] = (W[n][row][:] M_n)[c]   (k-major operand for the SYRK; W is track-major,
 //                   so this is a straight streaming pass), rhs[row] += Z[row] . q
-//   syrk            Sraw -= Zt^T Zt on the lower-triangular 128x128 tiles: FP64 FMA pipe, 8x8 register
-//                   tiles, cp.async double-buffered k-slabs, split-K with f64 RED epilogue
+//   (SYRK)          Sraw -= Zt^T Zt on the lower-triangular 128x128 tiles: tcgen05 INT8 Ozaki slices, csrc/syrk_i8.cu
 //   scale_damp      A = Dc Sraw Dc + diag(clamp(diag(Dc Hcc Dc)))/radius, constant parameters pinned
 //   cam_step / backsub_partial / point_step / cam_update   back-substitution and the candidate state
 #include <stddef.h>
-#include <stdlib.h>
 #include "common.cuh"
 
 namespace vgg {
@@ -214,222 +212,14 @@ __global__ void __launch_bounds__(128) z_build_kernel(int D, int N, int Dpad, si
 }
 
 // ------------------------------------------------------------------------------------------------
-// SYRK on lower-triangular tiles: C[bi,bj] -= Zt[:, bi]^T Zt[:, bj]
-constexpr int SY_BM = 128, SY_BK = 16, SY_THREADS = 256, SY_STAGES = 3;
-
-__global__ void __launch_bounds__(SY_THREADS) syrk_kernel(int Kpad, int Dpad, int k_per_split,
-                                                          const double* __restrict__ Zt, double* __restrict__ Cmat,
-                                                          ptrdiff_t mc_off, int fill_upper) {
-  extern __shared__ __align__(16) double sy_smem[];
-  // tile decode: blockIdx.x -> (bi >= bj)
-  int t = blockIdx.x;
-  int bi = (int)((sqrt(8.0 * t + 1.0) - 1.0) * 0.5);
-  while ((bi + 1) * (bi + 2) / 2 <= t) ++bi;
-  while (bi * (bi + 1) / 2 > t) --bi;
-  const int bj = t - bi * (bi + 1) / 2;
-  const bool diag = (bi == bj);
-  const int kbeg = blockIdx.y * k_per_split;
-  const int kend = min(Kpad, kbeg + k_per_split);
-  const int nslab = (kend - kbeg + SY_BK - 1) / SY_BK;
-  if (nslab <= 0) return;
-
-  double* As = sy_smem;                                   // [STAGES][BK][BM]
-  double* Bs = sy_smem + SY_STAGES * SY_BK * SY_BM;       // [STAGES][BK][BM]
-  const int tid = threadIdx.x;
-  const int ty = tid >> 4, tx = tid & 15;
-
-  auto load_slab = [&](int slab, int stage) {
-    const int k0 = kbeg + slab * SY_BK;
-    // each operand slab: BK x BM doubles = 1024 x 16B chunks; 256 threads x 4
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int chunk = tid + i * SY_THREADS;          // 0..1023
-      const int kk = chunk >> 6;                       // 64 chunks of 16 B per k-row
-      const int cc = (chunk & 63) * 2;
-      const size_t grow = (size_t)(k0 + kk) * Dpad;
-      cp_async16(As + (stage * SY_BK + kk) * SY_BM + cc, Zt + grow + bi * SY_BM + cc);
-      if (!diag) cp_async16(Bs + (stage * SY_BK + kk) * SY_BM + cc, Zt + grow + bj * SY_BM + cc);
-    }
-    cp_async_commit();
-  };
-
-  double acc[8][8];
-#pragma unroll
-  for (int i = 0; i < 8; ++i)
-#pragma unroll
-    for (int j = 0; j < 8; ++j) acc[i][j] = 0.0;
-
-  // prologue
-#pragma unroll
-  for (int s = 0; s < SY_STAGES - 1; ++s) {
-    if (s < nslab) load_slab(s, s);
-    else cp_async_commit();
-  }
-  for (int slab = 0; slab < nslab; ++slab) {
-    cp_async_wait<SY_STAGES - 2>();
-    __syncthreads();
-    {
-      const int nxt = slab + SY_STAGES - 1;
-      if (nxt < nslab) load_slab(nxt, nxt % SY_STAGES);
-      else cp_async_commit();
-    }
-    const int stage = slab % SY_STAGES;
-    const double* as = As + stage * SY_BK * SY_BM;
-    const double* bs = diag ? as : (Bs + stage * SY_BK * SY_BM);
-#pragma unroll
-    for (int kk = 0; kk < SY_BK; ++kk) {
-      double a[8], b[8];
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const double2 av = *reinterpret_cast<const double2*>(as + kk * SY_BM + ty * 2 + 32 * i);
-        a[2 * i] = av.x; a[2 * i + 1] = av.y;
-        const double2 bv = *reinterpret_cast<const double2*>(bs + kk * SY_BM + tx * 2 + 32 * i);
-        b[2 * i] = bv.x; b[2 * i + 1] = bv.y;
-      }
-#pragma unroll
-      for (int i = 0; i < 8; ++i)
-#pragma unroll
-        for (int j = 0; j < 8; ++j) acc[i][j] = fma(a[i], b[j], acc[i][j]);
-    }
-  }
-  cp_async_wait<0>();
-  // epilogue: C -= acc  (f64 RED; split-K partials and H_cc already in C)
-#pragma unroll
-  for (int i = 0; i < 8; ++i) {
-    const int r = bi * SY_BM + ty * 2 + (i & 1) + 32 * (i >> 1);
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      const int c = bj * SY_BM + tx * 2 + (j & 1) + 32 * (j >> 1);
-      if (acc[i][j] != 0.0) {
-        // row-major LOWER triangle (what csrc/chol.cu factors; in fabric mode one multimem op per element); the mirror
-        // only for the library factorisation A/B (fill_upper: cuSOLVER's fast path reads the column-major lower view)
-        if (!diag || c <= r) {
-          double* q = &Cmat[(size_t)r * Dpad + c];
-          ar_add(q, mc_off ? q + mc_off : nullptr, -acc[i][j]);
-        }
-        if (fill_upper && (!diag || c < r)) atomicAdd(&Cmat[(size_t)c * Dpad + r], -acc[i][j]);
-      }
-    }
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// Same SYRK on the FP64 tensor path: mma.sync.m8n8k4.f64 (SASS DMMA).  CTA tile 128x128, 8 warps as 4x2,
-// warp tile 32x64 = 4x8 MMA tiles (64 accumulator doubles per lane); operands k-major in shared memory with a
-// 136-double row stride so the four k-rows of a fragment load fall into disjoint bank halves.
-constexpr int SD_LDS = 136;
-
-__device__ __forceinline__ void dmma_m8n8k4(double& d0, double& d1, double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-               : "+d"(d0), "+d"(d1)
-               : "d"(a), "d"(b));
-}
-
-__global__ void __launch_bounds__(SY_THREADS) syrk_dmma_kernel(int Kpad, int Dpad, int k_per_split,
-                                                               const double* __restrict__ Zt,
-                                                               double* __restrict__ Cmat, ptrdiff_t mc_off,
-                                                               int fill_upper) {
-  extern __shared__ __align__(16) double sd_smem[];
-  int t = blockIdx.x;
-  int bi = (int)((sqrt(8.0 * t + 1.0) - 1.0) * 0.5);
-  while ((bi + 1) * (bi + 2) / 2 <= t) ++bi;
-  while (bi * (bi + 1) / 2 > t) --bi;
-  const int bj = t - bi * (bi + 1) / 2;
-  const bool diag = (bi == bj);
-  const int kbeg = blockIdx.y * k_per_split;
-  const int kend = min(Kpad, kbeg + k_per_split);
-  const int nslab = (kend - kbeg + SY_BK - 1) / SY_BK;
-  if (nslab <= 0) return;
-  double* As = sd_smem;                                      // [STAGES][BK][SD_LDS]
-  double* Bs = sd_smem + SY_STAGES * SY_BK * SD_LDS;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int wm = warp >> 1, wn = warp & 1;                   // 4 x 2 warps
-  const int g = lane >> 2, q = lane & 3;
-
-  auto load_slab = [&](int slab, int stage) {
-    const int k0 = kbeg + slab * SY_BK;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int chunk = tid + i * SY_THREADS;
-      const int kk = chunk >> 6;
-      const int cc = (chunk & 63) * 2;
-      const size_t grow = (size_t)(k0 + kk) * Dpad;
-      cp_async16(As + (stage * SY_BK + kk) * SD_LDS + cc, Zt + grow + bi * SY_BM + cc);
-      if (!diag) cp_async16(Bs + (stage * SY_BK + kk) * SD_LDS + cc, Zt + grow + bj * SY_BM + cc);
-    }
-    cp_async_commit();
-  };
-
-  double c[4][8][2];
-#pragma unroll
-  for (int i = 0; i < 4; ++i)
-#pragma unroll
-    for (int j = 0; j < 8; ++j) c[i][j][0] = c[i][j][1] = 0.0;
-
-#pragma unroll
-  for (int s = 0; s < SY_STAGES - 1; ++s) {
-    if (s < nslab) load_slab(s, s);
-    else cp_async_commit();
-  }
-  for (int slab = 0; slab < nslab; ++slab) {
-    cp_async_wait<SY_STAGES - 2>();
-    __syncthreads();
-    {
-      const int nxt = slab + SY_STAGES - 1;
-      if (nxt < nslab) load_slab(nxt, nxt % SY_STAGES);
-      else cp_async_commit();
-    }
-    const int stage = slab % SY_STAGES;
-    const double* as = As + stage * SY_BK * SD_LDS;
-    const double* bs = diag ? as : (Bs + stage * SY_BK * SD_LDS);
-#pragma unroll
-    for (int k4 = 0; k4 < SY_BK / 4; ++k4) {
-      double a[4], b[8];
-      const double* arow = as + (k4 * 4 + q) * SD_LDS + wm * 32 + g;
-      const double* brow = bs + (k4 * 4 + q) * SD_LDS + wn * 64 + g;
-#pragma unroll
-      for (int i = 0; i < 4; ++i) a[i] = arow[i * 8];
-#pragma unroll
-      for (int j = 0; j < 8; ++j) b[j] = brow[j * 8];
-#pragma unroll
-      for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 8; ++j) dmma_m8n8k4(c[i][j][0], c[i][j][1], a[i], b[j]);
-    }
-  }
-  cp_async_wait<0>();
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int r = bi * SY_BM + wm * 32 + i * 8 + g;
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      const int cc = bj * SY_BM + wn * 64 + j * 8 + 2 * q;
-#pragma unroll
-      for (int h = 0; h < 2; ++h) {
-        const double v = c[i][j][h];
-        const int col = cc + h;
-        if (v != 0.0) {
-          if (!diag || col <= r) {
-            double* q = &Cmat[(size_t)r * Dpad + col];
-            ar_add(q, mc_off ? q + mc_off : nullptr, -v);
-          }
-          if (fill_upper && (!diag || col < r)) atomicAdd(&Cmat[(size_t)col * Dpad + r], -v);   // library A/B only
-        }
-      }
-    }
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// A (in place) = sc_i sc_j Sraw + diag; constant parameters pinned; b = sc * rhs.  Lower triangle only unless
-// fill_upper (library factorisation A/B, which reads the mirror).
+// A (in place) = sc_i sc_j Sraw + diag; constant parameters pinned; b = sc * rhs.  Lower triangle only.
 __global__ void scale_damp_kernel(int D, int Dpad, double* __restrict__ A, const double* __restrict__ rhs,
                                   const double* __restrict__ hdiag, const double* __restrict__ sc,
                                   const uint8_t* __restrict__ pconst, double radius, double min_diag, double max_diag,
-                                  double* __restrict__ bvec, int fill_upper) {
+                                  double* __restrict__ bvec) {
   const int j = blockIdx.x * blockDim.x + threadIdx.x;
   const int i = blockIdx.y;
-  if (j >= D || (!fill_upper && j > i)) return;
+  if (j > i) return;
   const bool ci = pconst[i] != 0, cj = pconst[j] != 0;
   double v;
   if (ci || cj) {
@@ -441,13 +231,12 @@ __global__ void scale_damp_kernel(int D, int Dpad, double* __restrict__ A, const
   A[(size_t)i * Dpad + j] = v;
   if (i == j) {
     // The scaled right-hand side also becomes row D of the matrix (in the workspace rhs IS row D, so this scales it in
-    // place; the library A/B wants it as column D = row D of its column-major view): the factorisation of the bordered
+    // place): the factorisation of the bordered
     // matrix [[A, b], [b^T, c]] = [[L, 0], [y^T, .]] leaves y = L^-1 b there, i.e. the forward substitution comes out
     // of the factorisation for free (csrc/ba_solve.cu).  c only has to exceed y^T y.
     const double b = ci ? 0.0 : rhs[i] * sc[i];
     bvec[i] = b;
-    if (fill_upper) A[(size_t)i * Dpad + D] = b;
-    else A[(size_t)D * Dpad + i] = b;
+    A[(size_t)D * Dpad + i] = b;
     if (i == 0) A[(size_t)D * Dpad + D] = 1e300;
   }
 }
@@ -654,45 +443,14 @@ int launch_z_transpose(int D, int N, int Dpad, const double* W, const double* M,
   VGG_LAUNCH_CHECK();
   return VGG_OK;
 }
-// 0 (default): the reduced system is kept as a row-major LOWER triangle (csrc/chol.cu); 1: both triangles, for the
-// library factorisation A/B (set by csrc/ba_solve.cu from VGG_CHOL)
-int g_fill_upper = 0;
-
 // reduce-scatter destinations of the running multi-GPU solve (set per iteration by csrc/ba_solve.cu; world <= 1: off)
 FabricDev g_fabric_dev = {0, 0, {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr}};
 
-int launch_syrk(int Kpad, int Dpad, const double* Zt, double* Cmat, ptrdiff_t mc_off, cudaStream_t st) {
-  const int nb = Dpad / SY_BM;
-  const int ntiles = nb * (nb + 1) / 2;
-  const int nslab = Kpad / SY_BK;
-  // split K so that the grid covers the 148 SMs a few times over
-  int splits = (148 * 3 + ntiles - 1) / ntiles;
-  if (splits < 1) splits = 1;
-  if (splits > nslab) splits = nslab;
-  int slabs_per = (nslab + splits - 1) / splits;
-  splits = (nslab + slabs_per - 1) / slabs_per;
-  const size_t smem = sizeof(double) * 2 * SY_STAGES * SY_BK * SY_BM;
-  const size_t smem_d = sizeof(double) * 2 * SY_STAGES * SY_BK * SD_LDS;
-  static bool attr_set = false;
-  static int use_dmma = 0;
-  if (!attr_set) {
-    VGG_CUDA_CHECK(cudaFuncSetAttribute(syrk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    VGG_CUDA_CHECK(cudaFuncSetAttribute(syrk_dmma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_d));
-    const char* e = getenv("VGG_SYRK_DMMA");
-    use_dmma = (e && e[0] == '0') ? 0 : 1;     // DMMA is the default (r01 A/B: 3.1 ms -> 2.4 ms at C3); VGG_SYRK_DMMA=0 selects the DFMA kernel
-    attr_set = true;
-  }
-  dim3 grid(ntiles, splits);
-  if (use_dmma) syrk_dmma_kernel<<<grid, SY_THREADS, smem_d, st>>>(Kpad, Dpad, slabs_per * SY_BK, Zt, Cmat, mc_off, g_fill_upper);
-  else syrk_kernel<<<grid, SY_THREADS, smem, st>>>(Kpad, Dpad, slabs_per * SY_BK, Zt, Cmat, mc_off, g_fill_upper);
-  VGG_LAUNCH_CHECK();
-  return VGG_OK;
-}
 int launch_scale_damp(int D, int Dpad, double* A, const double* rhs, const double* hdiag, const double* sc,
                       const uint8_t* pconst, double radius, double min_diag, double max_diag, double* bvec,
                       cudaStream_t st) {
   dim3 grid((D + 255) / 256, D);
-  scale_damp_kernel<<<grid, 256, 0, st>>>(D, Dpad, A, rhs, hdiag, sc, pconst, radius, min_diag, max_diag, bvec, g_fill_upper);
+  scale_damp_kernel<<<grid, 256, 0, st>>>(D, Dpad, A, rhs, hdiag, sc, pconst, radius, min_diag, max_diag, bvec);
   VGG_LAUNCH_CHECK();
   return VGG_OK;
 }

@@ -3,7 +3,6 @@
 // iteration on one stream and ONE small device->host read (accept/reject scalars); track shards on
 // other GPUs join through the caller's all-reduce hook (NCCL over NVLink, see vggsfm_b200/dist.py).
 #include <cublas_v2.h>
-#include <cusolverDn.h>
 #include <math.h>
 #include <stdlib.h>
 #include <string.h>
@@ -35,7 +34,6 @@ int launch_assemble_hc(int S, int dc, int ns, int KR, int Dpad, const double* ca
                        double* Sraw, double* rhs, double* hdiag, double* gvec, ptrdiff_t mc_off, cudaStream_t st);
 int launch_z_transpose(int D, int N, int Dpad, const double* W, const double* M, const double* q, double* Zt,
                        double* rhs, ptrdiff_t mc_off, cudaStream_t st, unsigned long long* amax);
-int launch_syrk(int Kpad, int Dpad, const double* Zt, double* Cmat, ptrdiff_t mc_off, cudaStream_t st);
 size_t syrk_i8_workspace_bytes(int Kpad, int Dpad, int slices);
 int launch_syrk_i8(int Kpad, int Dpad, const double* Zt, double* Cmat, ptrdiff_t mc_off, int slices, void* ws,
                    size_t ws_bytes, cudaStream_t st, bool amax_ready);
@@ -57,12 +55,9 @@ int launch_extract_gvec(int S, int dc, int ns, int KR, const double* camrec, con
 int launch_gradmax(int D, int N, const double* gvec, const uint8_t* pconst, const double* g_p,
                    const uint8_t* point_const, double* scal, cudaStream_t st);
 
-size_t trsv_workspace_ints(int n);
-int launch_trsv_upper(int n, int lda, const double* A, const double* y, size_t y_stride, double* x, int* flags, int epoch,
-                      cudaStream_t st);
+int launch_trsv_upper(int n, int lda, const double* A, const double* y, size_t y_stride, double* x, cudaStream_t st);
 size_t chol_workspace_doubles(int n);
 int chol_lower_inplace(int n, int lda, double* A, double* Ldiag, int* info, cudaStream_t st);
-extern int g_fill_upper;       // csrc/ba_schur.cu: 1 = also write the mirror triangle (library factorisation A/B)
 extern FabricDev g_fabric_dev; // csrc/ba_schur.cu: reduce-scatter destinations read by the SYRK epilogue
 int launch_fabric_barrier(const FabricDev& fd, size_t flags_off, unsigned long long epoch, int* err, cudaStream_t st);
 int launch_fabric_gather(const FabricDev& fd, int nrows, int nmat, int ncols_vec, int lda, cudaStream_t st);
@@ -70,13 +65,13 @@ int launch_fabric_allreduce(const FabricDev& fd, size_t flags_off, size_t mail_o
                             unsigned long long epoch, double* vec, int count, int max_slot, int* err, cudaStream_t st);
 
 // gathers the accept/reject scalars into one 24-double record so the host reads them with ONE copy:
-// [0..7] = scal[0..7], [8..15] = small[0..7], [16] = potrf info, [17] = potrs info, [18] = |x|^2
+// [0..7] = scal[0..7], [8..15] = small[0..7], [16] = factorisation info, [18] = |x|^2, [19] = fabric barrier timeout
 __global__ void pack_scalars_kernel(const double* __restrict__ scal, const double* __restrict__ small,
                                     const int* __restrict__ info, double* __restrict__ out) {
   const int i = threadIdx.x;
   if (i < 8) out[i] = scal[i];
   else if (i < 16) out[i] = small[i - 8];
-  else if (i < 18) out[i] = (double)info[i - 16];
+  else if (i == 16) out[i] = (double)info[0];       // chol.cu: non-positive pivot
   else if (i == 18) out[i] = scal[8];              // |x|^2 (xnorm_kernel), 0 unless parameter_tolerance > 0
   else if (i == 19) out[i] = (double)info[2];      // a cross-rank barrier of csrc/fabric.cu timed out
 }
@@ -171,34 +166,19 @@ struct Layout {
   double *small;     // [8 scalars | gvec_candidate Dpad]           (one small all-reduce)
   double *scal;      // [16]
   double *packed;    // [24] scalars gathered for the host
-  double *potrf_work;
   double *chol_diag;
   int *dev_info;
-  int *trsv_flags;
   uint8_t* oz_ws;    // int8 slices + scales of the tensor-core SYRK (csrc/syrk_i8.cu)
   size_t oz_bytes;
-  size_t potrf_lwork;
   size_t bytes;
 };
 
-// The Schur SYRK runs on the tensor cores by default (tcgen05 INT8 Ozaki slices, csrc/syrk_i8.cu: r01 A/B at C3
-// 2.46 ms -> 1.10 ms per iteration, 238 -> 348 it/s, same iterates).  VGG_SYRK=ozaki:N picks 3..7 slices (default 7 =
-// 54 fractional bits, FP64-equivalent); VGG_SYRK=fp64 selects the FP64-pipe kernels (DMMA / DFMA).
-static int syrk_i8_slices() {
-  static int slices = -1;
-  if (slices < 0) {
-    slices = 7;
-    const char* e = getenv("VGG_SYRK");
-    if (e && strncmp(e, "ozaki", 5) == 0) {
-      if (e[5] == ':' && e[6] >= '3' && e[6] <= '7') slices = e[6] - '0';
-    } else if (e && e[0]) {
-      slices = 0;
-    }
-  }
-  return slices;
-}
+// The Schur SYRK runs on the tensor cores (tcgen05 INT8 Ozaki slices, csrc/syrk_i8.cu) with 7 slices = 54 fractional
+// bits, FP64-equivalent.  It replaced the FP64-pipe DMMA / DFMA kernels: 2.46 ms -> 1.10 ms per iteration at C3 on a
+// B200, same iterates (profiles/r01_*).
+constexpr int kSyrkSlices = 7;
 
-static int make_layout(int S, int N, int model, int mode, void* base, size_t cap, size_t potrf_lwork, Layout* L) {
+static int make_layout(int S, int N, int model, int mode, void* base, size_t cap, Layout* L) {
   int dc, ns, KR;
   if (dims_of(model, mode, &dc, &ns, &KR) != VGG_OK) {
     set_error("bad camera_model/intr_mode");
@@ -233,12 +213,9 @@ static int make_layout(int S, int N, int model, int mode, void* base, size_t cap
   L->small = c.take<double>(8 + (size_t)L->Dpad);
   L->scal = c.take<double>(16);
   L->packed = c.take<double>(32);
-  L->potrf_lwork = potrf_lwork;
-  L->potrf_work = c.take<double>(potrf_lwork);
   L->chol_diag = c.take<double>(chol_workspace_doubles(L->D + 1));
   L->dev_info = c.take<int>(4);
-  L->trsv_flags = c.take<int>(trsv_workspace_ints(L->D));
-  L->oz_bytes = syrk_i8_workspace_bytes(L->Kpad, L->Dpad, 7);
+  L->oz_bytes = syrk_i8_workspace_bytes(L->Kpad, L->Dpad, kSyrkSlices);
   c.off = align_up(c.off, 1024);
   L->oz_ws = c.take<uint8_t>(L->oz_bytes);
   L->bytes = align_up(c.off, 256);
@@ -249,44 +226,12 @@ static int make_layout(int S, int N, int model, int mode, void* base, size_t cap
   return VGG_OK;
 }
 
-static cusolverDnHandle_t get_cusolver() {
-  static thread_local cusolverDnHandle_t h = nullptr;
-  if (!h) {
-    if (cusolverDnCreate(&h) != CUSOLVER_STATUS_SUCCESS) h = nullptr;
-  }
-  return h;
-}
-
 static cublasHandle_t get_cublas() {
   static thread_local cublasHandle_t h = nullptr;
   if (!h) {
     if (cublasCreate(&h) != CUBLAS_STATUS_SUCCESS) h = nullptr;
   }
   return h;
-}
-
-// Doubles of device scratch the factorisation needs at order D+1 (bordered system): the larger of the 32-bit
-// cusolverDnDpotrf and the 64-bit cusolverDnXpotrf requirement, so one carved region serves either call.
-static int potrf_lwork(int D, int Dpad, size_t* lwork) {
-  cusolverDnHandle_t h = get_cusolver();
-  if (!h) {
-    set_error("cusolverDnCreate failed");
-    return VGG_ESOLVER;
-  }
-  int lw = 0;
-  if (cusolverDnDpotrf_bufferSize(h, CUBLAS_FILL_MODE_LOWER, D + 1, nullptr, Dpad, &lw) != CUSOLVER_STATUS_SUCCESS) {
-    set_error("cusolverDnDpotrf_bufferSize failed");
-    return VGG_ESOLVER;
-  }
-  size_t need = (size_t)lw;
-  static thread_local cusolverDnParams_t xp = nullptr;
-  if (!xp) cusolverDnCreateParams(&xp);
-  size_t db = 0, hb = 0;
-  if (xp && cusolverDnXpotrf_bufferSize(h, xp, CUBLAS_FILL_MODE_LOWER, D + 1, CUDA_R_64F, nullptr, Dpad, CUDA_R_64F, &db, &hb) ==
-                CUSOLVER_STATUS_SUCCESS)
-    need = need > (db + 7) / 8 ? need : (db + 7) / 8;
-  *lwork = need;
-  return VGG_OK;
 }
 
 // Layout of the symmetric allocation of fabric v2 (doubles): two copies of the reduced system (iteration parity, so a
@@ -337,7 +282,6 @@ extern BandDev g_band_dev;                    // csrc/ba_schur.cu: device tables
 struct SolveGuard {
   ~SolveGuard() {
     g_fabric_dev.world = 0;
-    g_fill_upper = 0;
     g_syrk_kb_ranges.clear();
     g_chol_band_end.clear();
     g_chol_arrow_blk = 0;
@@ -512,13 +456,9 @@ static int schur_build(const Layout& L, const BlockSet& b, const uint8_t* point_
   // fabric mode: every rank's copy must be zero before anyone's multimem reductions land in it
   if (mc_off && barrier && (rc = (*barrier)())) return rc;
   if ((rc = launch_assemble_hc(L.S, L.dc, L.ns, L.KR, L.Dpad, b.camrec, b.shared, Sraw, rhs, hdiag, gvec, mc_off, st))) return rc;
-  const int oz = L.oz_bytes ? syrk_i8_slices() : 0;
-  if (oz && (rc = syrk_i8_reset_amax(L.oz_ws, L.Dpad, st))) return rc;
-  if ((rc = launch_z_transpose(L.D, L.N, L.Dpad, b.W, L.M, L.q, L.Zt, rhs, mc_off, st, oz ? syrk_i8_amax(L.oz_ws) : nullptr)))
-    return rc;
-  if (oz) rc = launch_syrk_i8(L.Kpad, L.Dpad, L.Zt, Sraw, mc_off, oz, L.oz_ws, L.oz_bytes, st, true);
-  else rc = launch_syrk(L.Kpad, L.Dpad, L.Zt, Sraw, mc_off, st);
-  if (rc) return rc;
+  if ((rc = syrk_i8_reset_amax(L.oz_ws, L.Dpad, st))) return rc;
+  if ((rc = launch_z_transpose(L.D, L.N, L.Dpad, b.W, L.M, L.q, L.Zt, rhs, mc_off, st, syrk_i8_amax(L.oz_ws)))) return rc;
+  if ((rc = launch_syrk_i8(L.Kpad, L.Dpad, L.Zt, Sraw, mc_off, kSyrkSlices, L.oz_ws, L.oz_bytes, st, true))) return rc;
   // ... and all reductions must have landed before anyone reads its copy
   if (mc_off && barrier && (rc = (*barrier)())) return rc;
   return VGG_OK;
@@ -566,12 +506,8 @@ int vgg_ba_workspace_bytes(int S, int N, int camera_model, int intr_mode, size_t
     set_error("bad camera_model/intr_mode");
     return VGG_EINVAL;
   }
-  const int D = S * dc + ns;
-  size_t lwork = 0;
-  int rc = potrf_lwork(D, (int)align_up((size_t)D + 2, 128), &lwork);
-  if (rc) return rc;
   Layout L;
-  rc = make_layout(S, N, camera_model, intr_mode, nullptr, 0, lwork, &L);
+  const int rc = make_layout(S, N, camera_model, intr_mode, nullptr, 0, &L);
   if (rc) return rc;
   *bytes = L.bytes;
   return VGG_OK;
@@ -591,13 +527,8 @@ int vgg_ba_schur(const vgg_ba_problem* prob, const double* camrec, const double*
   VGG_REQUIRE(prob && workspace && Sraw && rhs, "null pointer");
   cudaStream_t st = (cudaStream_t)stream;
   g_launch_count = 0;
-  size_t lwork = 0;
-  int dc, ns;
-  dims_of(prob->camera_model, prob->intr_mode, &dc, &ns, nullptr);
-  int rc = potrf_lwork(prob->S * dc + ns, (int)align_up((size_t)(prob->S * dc + ns) + 2, 128), &lwork);
-  if (rc) return rc;
   Layout L;
-  rc = make_layout(prob->S, prob->N, prob->camera_model, prob->intr_mode, workspace, ws_bytes, lwork, &L);
+  int rc = make_layout(prob->S, prob->N, prob->camera_model, prob->intr_mode, workspace, ws_bytes, &L);
   if (rc) return rc;
   BlockSet b;
   b.cost = nullptr;
@@ -681,17 +612,9 @@ int vgg_ba_solve_fabric(const vgg_ba_problem* prob, const vgg_ba_options* opt_in
     return VGG_EINVAL;
   }
   const int D = S * dc + ns;
-  size_t lwork = 0;
-  int rc = potrf_lwork(D, (int)align_up((size_t)D + 2, 128), &lwork);
-  if (rc) return rc;
   Layout L;
-  rc = make_layout(S, N, prob->camera_model, prob->intr_mode, workspace, ws_bytes, lwork, &L);
+  int rc = make_layout(S, N, prob->camera_model, prob->intr_mode, workspace, ws_bytes, &L);
   if (rc) return rc;
-  cusolverDnHandle_t cs = get_cusolver();
-  if (cusolverDnSetStream(cs, st) != CUSOLVER_STATUS_SUCCESS) {
-    set_error("cusolverDnSetStream failed");
-    return VGG_ESOLVER;
-  }
   const size_t ar_count = (size_t)D * L.Dpad + 3 * (size_t)L.Dpad;
   // fabric mode: the reduced system lives in symmetric (peer-mapped) memory and is reduced by multimem operations
   // issued from the producing kernels; mc_off is the distance from a local address to its multicast twin
@@ -707,8 +630,7 @@ int vgg_ba_solve_fabric(const vgg_ba_problem* prob, const vgg_ba_options* opt_in
     // barriers and small all-reduces through the host hook) for A/B
     static const bool want_v2 = [] { const char* e = getenv("VGG_FABRIC"); return !(e && e[0] == '1'); }();
     const FabricLayout lay = fabric_layout(D, L.Dpad);
-    if (want_v2 && fabric->world > 1 && fabric->world <= 8 && fabric->peer_base[0] && fabric->total_doubles >= lay.total &&
-        L.oz_bytes && syrk_i8_slices() > 0) {
+    if (want_v2 && fabric->world > 1 && fabric->world <= 8 && fabric->peer_base[0] && fabric->total_doubles >= lay.total) {
       fab2.on = true;
       fab2.lay = lay;
       fab2.base.world = fabric->world;
@@ -720,7 +642,7 @@ int vgg_ba_solve_fabric(const vgg_ba_problem* prob, const vgg_ba_options* opt_in
       VGG_REQUIRE(allreduce, "fabric v1 needs the hook for its barrier (op 2)");
     }
   }
-  if (L.oz_bytes && (rc = compute_band_hint(prob, dc, D, L.Dpad, L.Kpad, allreduce != nullptr || fabric != nullptr, st))) return rc;
+  if ((rc = compute_band_hint(prob, dc, D, L.Dpad, L.Kpad, allreduce != nullptr || fabric != nullptr, st))) return rc;
   if (g_band_dev.fg_tracks) {
     // the kernels skip the (track chunk, frame group) regions no observation falls into: their W blocks must read as zero
     const size_t w_doubles = (size_t)N * (size_t)(D + (D & 1)) * 3;
@@ -741,15 +663,6 @@ int vgg_ba_solve_fabric(const vgg_ba_problem* prob, const vgg_ba_options* opt_in
     if (allreduce) return allreduce(ar_user, vec, count, op, st);
     return VGG_OK;
   };
-  // factorisation: 2 = csrc/chol.cu (default), 0 = cuSOLVER Xpotrf (VGG_CHOL=lib), 1 = cuSOLVER Dpotrf (VGG_CHOL=legacy)
-  static const int chol_mode = [] {
-    const char* e = getenv("VGG_CHOL");
-    if (!e || !e[0] || e[0] == 'o') return 2;
-    return (e[0] == 'l' && e[1] == 'e') ? 1 : 0;
-  }();
-  const int cm = mc_off ? 2 : chol_mode;           // fabric mode reduces the lower triangle only
-  g_fill_upper = cm != 2;
-
   EventPair evs;
   VGG_CUDA_CHECK(cudaEventCreate(&evs.a));
   VGG_CUDA_CHECK(cudaEventCreate(&evs.b));
@@ -858,76 +771,32 @@ int vgg_ba_solve_fabric(const vgg_ba_problem* prob, const vgg_ba_options* opt_in
     if ((rc = launch_scale_damp(D, L.Dpad, Sraw, rhs, hdiag, L.sc_c, prob->param_const, radius, opt.min_lm_diagonal,
                                 opt.max_lm_diagonal, L.bvec, st)))
       return rc;
-    // Factor the reduced system.  Default: the in-repo blocked Cholesky (csrc/chol.cu) on the row-major LOWER triangle,
-    // of the BORDERED matrix of order D+1 -- scale_damp put the scaled right-hand side into row D, so the factorisation
-    // leaves y = L^-1 b there (and, mirrored like every panel, in column D): the forward substitution costs nothing and
-    // only the backward substitution L^T x = y remains.  VGG_CHOL=lib (cuSOLVER 64-bit potrf on the column-major LOWER
-    // view, r01 default, 1.05 ms at n = 2403) and VGG_CHOL=legacy (32-bit potrf) are kept for A/B; they need the mirror
-    // triangle (g_fill_upper) and are not available in fabric mode.
-    const int nfac = D + 1;
-    if (cm == 2) {
-      if ((rc = chol_lower_inplace(nfac, L.Dpad, Sraw, L.chol_diag, L.dev_info, st))) return rc;
-    } else if (cm == 0) {
-      static thread_local cusolverDnParams_t xp = nullptr;
-      static thread_local void* xdev_fallback = nullptr;
-      static thread_local void* xhost = nullptr;
-      static thread_local size_t xdev_b = 0, xhost_b = 0;
-      if (!xp) cusolverDnCreateParams(&xp);
-      size_t db = 0, hb = 0;
-      if (cusolverDnXpotrf_bufferSize(cs, xp, CUBLAS_FILL_MODE_LOWER, nfac, CUDA_R_64F, Sraw, L.Dpad, CUDA_R_64F, &db, &hb) !=
-          CUSOLVER_STATUS_SUCCESS) {
-        set_error("cusolverDnXpotrf_bufferSize failed");
-        return VGG_ESOLVER;
-      }
-      // device scratch comes out of the caller's workspace (sized by potrf_lwork); the cudaMalloc below only runs if
-      // a library version asks for more at solve time than it reported when the workspace was sized
-      void* xdev = L.potrf_work;
-      if (db > L.potrf_lwork * sizeof(double)) {
-        if (db > xdev_b) { if (xdev_fallback) cudaFree(xdev_fallback); VGG_CUDA_CHECK(cudaMalloc(&xdev_fallback, db)); xdev_b = db; }
-        xdev = xdev_fallback;
-      }
-      if (hb > xhost_b) { free(xhost); xhost = malloc(hb); xhost_b = hb; }
-      if (cusolverDnXpotrf(cs, xp, CUBLAS_FILL_MODE_LOWER, nfac, CUDA_R_64F, Sraw, L.Dpad, CUDA_R_64F, xdev, db, xhost, hb,
-                           L.dev_info) != CUSOLVER_STATUS_SUCCESS) {
-        set_error("cusolverDnXpotrf failed to launch");
-        return VGG_ESOLVER;
-      }
-      g_launch_count += 1;
-    } else {
-      if (cusolverDnDpotrf(cs, CUBLAS_FILL_MODE_LOWER, nfac, Sraw, L.Dpad, L.potrf_work, (int)L.potrf_lwork, L.dev_info) !=
-          CUSOLVER_STATUS_SUCCESS) {
-        set_error("cusolverDnDpotrf failed to launch");
-        return VGG_ESOLVER;
-      }
-      g_launch_count += 1;
-    }
-    // Backward substitution on U = L^T (the row-major upper triangle in every mode), y = column D of the buffer.
+    // Factor the reduced system: the in-repo blocked Cholesky (csrc/chol.cu) on the row-major LOWER triangle of the
+    // BORDERED matrix of order D+1 -- scale_damp put the scaled right-hand side into row D, so the factorisation leaves
+    // y = L^-1 b there (and, mirrored like every panel, in column D): the forward substitution costs nothing and only the
+    // backward substitution L^T x = y remains.  It replaced cuSOLVER potrf (1.145 ms vs 0.88 ms at n = 2403 on a B200,
+    // profiles/r02_*).
+    if ((rc = chol_lower_inplace(D + 1, L.Dpad, Sraw, L.chol_diag, L.dev_info, st))) return rc;
+    // Backward substitution on U = L^T (the row-major upper triangle), y = column D of the buffer.
     const double* dcs = L.bvec;
     size_t dcs_stride = 1;
-    {
-      static const bool lib_trsv = [] {
-        const char* e = getenv("VGG_TRSV");
-        return e && e[0] == 'c';                     // VGG_TRSV=cublas keeps the library call for A/B
-      }();
-      VGG_CUDA_CHECK(cudaMemsetAsync(L.dev_info + 1, 0, sizeof(int), st));
-      if (lib_trsv || D > 7000) {                     // own kernel: one co-resident wave of D/64 CTAs
-        cublasHandle_t cb = get_cublas();
-        if (!cb || cublasSetStream(cb, st) != CUBLAS_STATUS_SUCCESS) {
-          set_error("cublasCreate / cublasSetStream failed");
-          return VGG_ESOLVER;
-        }
-        if (cublasDtrsv(cb, CUBLAS_FILL_MODE_LOWER, CUBLAS_OP_T, CUBLAS_DIAG_NON_UNIT, D, Sraw, L.Dpad, Sraw + D, L.Dpad) !=
-            CUBLAS_STATUS_SUCCESS) {
-          set_error("cublasDtrsv failed to launch");
-          return VGG_ESOLVER;
-        }
-        g_launch_count += 1;
-        dcs = Sraw + D;
-        dcs_stride = (size_t)L.Dpad;
-      } else {
-        // own backward substitution (csrc/trsv.cu): one launch, block rows chained through flags
-        if ((rc = launch_trsv_upper(D, L.Dpad, Sraw, Sraw + D, (size_t)L.Dpad, L.bvec, L.trsv_flags, 1, st))) return rc;
+    if (D > 7000) {                                   // own kernel needs one co-resident wave of D/64 CTAs
+      cublasHandle_t cb = get_cublas();
+      if (!cb || cublasSetStream(cb, st) != CUBLAS_STATUS_SUCCESS) {
+        set_error("cublasCreate / cublasSetStream failed");
+        return VGG_ESOLVER;
       }
+      if (cublasDtrsv(cb, CUBLAS_FILL_MODE_LOWER, CUBLAS_OP_T, CUBLAS_DIAG_NON_UNIT, D, Sraw, L.Dpad, Sraw + D, L.Dpad) !=
+          CUBLAS_STATUS_SUCCESS) {
+        set_error("cublasDtrsv failed to launch");
+        return VGG_ESOLVER;
+      }
+      g_launch_count += 1;
+      dcs = Sraw + D;
+      dcs_stride = (size_t)L.Dpad;
+    } else {
+      // own backward substitution (csrc/trsv.cu): one launch, block rows chained through the solution vector
+      if ((rc = launch_trsv_upper(D, L.Dpad, Sraw, Sraw + D, (size_t)L.Dpad, L.bvec, st))) return rc;
     }
     if ((rc = launch_cam_step(D, dcs, dcs_stride, L.sc_c, hdiag, gvec, prob->param_const, radius, opt.min_lm_diagonal,
                               opt.max_lm_diagonal, L.d_c, L.scal, st)))
@@ -976,7 +845,6 @@ int vgg_ba_solve_fabric(const vgg_ba_problem* prob, const vgg_ba_options* opt_in
       VGG_LAUNCH_CHECK();
     }
     if ((rc = read_scalars())) return rc;
-    const int h_info[2] = {(int)h_scal[16], (int)h_scal[17]};
 
     const double c_cost = h_scal[8];
     const double quad = h_scal[0] + h_scal[9];
@@ -986,7 +854,7 @@ int vgg_ba_solve_fabric(const vgg_ba_problem* prob, const vgg_ba_options* opt_in
       set_error("fabric barrier timed out: a peer rank did not arrive");
       return VGG_ECUDA;
     }
-    const bool solver_bad = h_info[0] != 0 || h_info[1] != 0 || h_scal[7] > 0 || h_scal[11] > 0;
+    const bool solver_bad = h_scal[16] != 0.0 || h_scal[7] > 0 || h_scal[11] > 0;
     double* tr = trace ? trace + (size_t)(it - 1) * 8 : nullptr;
     if (tr) {
       tr[0] = it; tr[1] = cost; tr[2] = c_cost; tr[3] = model_change; tr[4] = 0; tr[5] = radius; tr[6] = step_norm; tr[7] = 0;

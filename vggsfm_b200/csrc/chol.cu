@@ -12,10 +12,11 @@
 //   chol_update_kernel  A22 -= P P^T on 64x64 tiles with mma.sync.m8n8k4.f64 (SASS DMMA) for block columns >= k+2, on a
 //                       low-priority side stream; one K half of both operands in shared memory at a time (68 KB) so that
 //                       its CTAs run NEXT TO the panel CTAs of the following step (152 KB) on the same SMs.
-// The whole launch sequence is captured once per (matrix, order) into a CUDA graph.  Switches for A/B runs:
-// VGG_CHOL_FUSE=0 (separate critical-path update kernel + panel on a side stream, the first r02 schedule),
-// VGG_CHOL_LOOKAHEAD=0 (everything in program order), VGG_CHOL_GRAPH=0, VGG_CHOL_LEAF=0.
-#include <stdlib.h>
+// The whole launch sequence is captured once per (matrix, order) into a CUDA graph.  Matrices of fewer than three
+// panels (n <= 256) run in program order instead: update, then the next panel, all on the caller's stream.
+// Measured slower on a B200 and removed (profiles/README.md): the first r02 schedule (a separate critical-path update
+// kernel with the next panel on a side stream), a persistent trailing-update kernel (0.920 vs 0.890 ms at n = 2403) and
+// the one-pivot-per-step 8x8 leaf.
 #include <algorithm>
 #include <map>
 #include <vector>
@@ -65,14 +66,13 @@ __device__ __forceinline__ double fast_rsqrt(double p) {
 }
 constexpr double CHOL_PMIN = 2.2250738585072014e-308;      // smallest normal double: pivots below it count as non-positive
 
-// LEAF selects the 8x8 leaf (0: one pivot per step, 1: two pivots per step); PROBE adds clock64 phase counters for
-// tools/microbench.py chol128 (threads 0 and 32 = warp 0 / warp 1; prof[warp][phase], see the MARK sites).
+// PROBE adds clock64 phase counters for tools/microbench.py chol128 (threads 0 and 32 = warp 0 / warp 1; prof[warp][phase], see the MARK sites).
 //
 // xr (0 or C_RPC) extra rows stored right below the block (rows 128 .. 128+xr-1 of Ls) ride along: they take part in the
 // micro-panel solves and in the rank-8 / rank-32 updates, so when the block is factored they hold X = A_ik L^-T -- the
 // panel rows this CTA owns -- with no separate triangular solve afterwards (r02: that solve was a 128-step
 // multiply/shuffle/FMA chain, ~3 us after every POTRF128, plus a transposing pass over the block to feed it).
-template <int LEAF, bool PROBE>
+template <bool PROBE>
 __device__ __forceinline__ int cta_chol128(double* Ls, double* dinv, int* fail_sm, int tid, int xr,
                                            long long* prof = nullptr) {
   const int lane = tid & 31, warp = tid >> 5;
@@ -107,7 +107,7 @@ __device__ __forceinline__ int cta_chol128(double* Ls, double* dinv, int* fail_s
   // back to the sequential formula (warp-uniform branch).  A shuffle-free variant (every lane holds the whole
   // 36-element triangle) measured SLOWER: panel 51.6 vs 48.6 us -- 36 broadcast loads + 64 predicated stores per leaf
   // cost more than the shuffles they replace.
-  auto leaf1 = [&](int c0) {
+  auto leaf = [&](int c0) {
     double a[8];
     const int r = c0 + (lane & 7);
 #pragma unroll
@@ -168,49 +168,6 @@ __device__ __forceinline__ int cta_chol128(double* Ls, double* dinv, int* fail_s
       for (int c = 0; c < 8; ++c) Lh[lane * 8 + c] = (c < lane) ? a[c] * mydinv : 0.0;
     }
     if (lane == 0 && fail && *fail_sm == 0) *fail_sm = fail;
-  };
-  // one pivot per step (the r02 default until the two-pivot leaf; kept for A/B through the probe)
-  auto leaf0 = [&](int c0) {
-    double a[8];
-    const int r = c0 + (lane & 7);
-#pragma unroll
-    for (int c = 0; c < 8; c += 2) {
-      const double2 v = *reinterpret_cast<const double2*>(Ls + r * CLD + c0 + c);
-      a[c] = v.x;
-      a[c + 1] = v.y;
-    }
-    int fail = 0;
-    double mydinv = 1.0;
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      const double pj = __shfl_sync(0xffffffffu, a[j], j);
-      double inv = fast_rsqrt(pj);
-      if (!(pj >= CHOL_PMIN)) {                               // uniform; tested in the shadow of the rsqrt chain
-        if (fail == 0) fail = c0 + j + 1;
-        inv = 1.0;
-      }
-      a[j] = a[j] * inv;                                      // lane j: pj * inv = sqrt(pj)
-      if (lane == j) {
-        dinv[c0 + j] = inv;
-        mydinv = inv;
-      }
-#pragma unroll
-      for (int c = j + 1; c < 8; ++c) {
-        const double lc = __shfl_sync(0xffffffffu, a[j], c);
-        if (lane >= c) a[c] = fma(-a[j], lc, a[c]);
-      }
-    }
-    if (lane < 8) {
-#pragma unroll
-      for (int c = 0; c < 8; ++c) Ls[r * CLD + c0 + c] = (c <= lane) ? a[c] : 0.0;
-#pragma unroll
-      for (int c = 0; c < 8; ++c) Lh[lane * 8 + c] = (c < lane) ? a[c] * mydinv : 0.0;
-    }
-    if (lane == 0 && fail && *fail_sm == 0) *fail_sm = fail;
-  };
-  auto leaf = [&](int c0) {
-    if constexpr (LEAF == 0) leaf0(c0);
-    else leaf1(c0);
   };
   // C[r][j] -= sum_k L[r][c0+k] L[j][c0+k] for j = jb, jb+js, ... <= jend (two columns in flight)
   auto row_update = [&](int r, int c0, int jb, int js, int jend) {
@@ -418,7 +375,6 @@ __device__ __forceinline__ int cta_chol128(double* Ls, double* dinv, int* fail_s
 }
 
 // one-CTA probe: factor a 128 x 128 block `reps` times (reloading it each time), report the cycles of the last pass
-template <int LEAF>
 __global__ void __launch_bounds__(C_THREADS, 1) chol128_probe_kernel(const double* __restrict__ A, double* __restrict__ L,
                                                                       long long* __restrict__ prof, int reps, int xr) {
   extern __shared__ __align__(16) double cp_smem[];
@@ -432,7 +388,7 @@ __global__ void __launch_bounds__(C_THREADS, 1) chol128_probe_kernel(const doubl
       cp_smem[(CB + (e >> 7)) * CLD + (e & 127)] = A[(CB - xr + (e >> 7)) * CB + (e & 127)];
     __syncthreads();
     const long long t0 = clock64();
-    cta_chol128<LEAF, true>(cp_smem, dinv, &fail_sm, tid, xr, prof);
+    cta_chol128<true>(cp_smem, dinv, &fail_sm, tid, xr, prof);
     __syncthreads();
     total = clock64() - t0;
   }
@@ -457,7 +413,6 @@ __global__ void __launch_bounds__(C_THREADS, 1) chol128_probe_kernel(const doubl
 constexpr int CHOL_SPIN_LIMIT = 1 << 22;
 constexpr int CHOL_INFO_STALLED = 0x7fffffff;
 
-template <int LEAF>
 __global__ void __launch_bounds__(C_THREADS, 1) chol_panel_kernel(int n, int lda, int k0, double* __restrict__ A,
                                                                    double* __restrict__ Ldiag /*[nblk][128*128]*/,
                                                                    int* __restrict__ info, int* __restrict__ flags,
@@ -494,7 +449,7 @@ __global__ void __launch_bounds__(C_THREADS, 1) chol_panel_kernel(int n, int lda
   cp_async_commit();
   cp_async_wait<0>();
   __syncthreads();
-  const int fail = cta_chol128<LEAF, false>(Ls, dinv, &fail_sm, tid, C_RPC);
+  const int fail = cta_chol128<false>(Ls, dinv, &fail_sm, tid, C_RPC);
   if (fail && blockIdx.x == 0 && tid == 0) atomicCAS(info, 0, k0 + fail);
   if (!solver) {
     // the last panel has no other CTA that could still be loading the block: its factor goes straight into place
@@ -621,40 +576,29 @@ __global__ void __launch_bounds__(C_THREADS, 1) chol_panel_kernel(int n, int lda
   }
 }
 
-// A[t0.., t0..] -= P P^T (lower part), P = A[t0.., k0..k0+127].  Tiles of TM rows x 64 columns, 8 warps.
-//   TM = 64 (trailing update off the critical path): tile (bi, bj), bj <= bi, warps 2x4, warp tile 32x16; mode 2 = tile
-//            columns >= 2, mode 0 = all; mode 3 = mode 2 with f64 REDs on tile columns 2 and 3 (the block column the
-//            fused panel kernel of the next step is adding into at the same time); mode 4 = tile columns 2 and 3 only
-//            (REDs), mode 5 = tile columns >= 4 (REDs on 4 and 5): the two halves of mode 3 with different deadlines.
-//   TM = 32 (mode 1, the next panel's 128 columns = tile columns 0 and 1, ON the critical path): twice as many CTAs so
-//            the ~140 tiles of a 2400-row matrix fill the 148 SMs with one short tile each; warps 1x8, warp tile 32x8.
+// A[t0.., t0..] -= P P^T (lower part), P = A[t0.., k0..k0+127].  64x64 tiles (bi, bj), bj <= bi, one per CTA, 8 warps
+// as 2x4, warp tile 32x16.  mode 0 = all tile columns; mode 4 = tile columns 2 and 3 only (block column k+2, which the
+// fused panel kernel of the next step is adding into at the same time: f64 REDs), mode 5 = tile columns >= 4 (REDs on 4
+// and 5): the two pieces of the trailing update with different deadlines.
 // Shared memory holds ONE K half (64 panel columns) of both operands at a time, row stride 68 doubles (fragment loads
 // conflict-free like stride 132): 68 KB per CTA instead of 135 KB, so an update CTA fits on an SM NEXT TO a panel CTA
 // (152 KB) and two or three fit on a free SM.  r02 launch list of the previous version (whole K resident, one CTA per
 // SM): the panel kernel's <= 143 latency-bound CTAs held their SMs for the whole step and the trailing update ran
 // after them, not beside them -- the factorisation took the SUM of all its kernels (0.90 ms).
 constexpr int CUD = 68;
-template <int TM>
 __global__ void __launch_bounds__(C_THREADS, 2) chol_update_kernel(int n, int lda, int k0, int t0, int mode,
                                                                     double* __restrict__ A, int band_end, int arrow_lo,
-                                                                    int all_red, int ntiles) {
-  constexpr int WN = TM == 64 ? 4 : 8;            // warps along the 64 tile columns
-  constexpr int NJ = 64 / WN / 8;                 // 8-column MMA tiles per warp: 2 or 1
+                                                                    int all_red) {
+  constexpr int TM = 64;                          // tile rows
+  constexpr int WN = 4;                           // warps along the 64 tile columns
+  constexpr int NJ = 64 / WN / 8;                 // 8-column MMA tiles per warp
   extern __shared__ __align__(16) double cu_smem[];
   double* As = cu_smem;                         // [TM][CUD]
   double* Bs = cu_smem + TM * CUD;              // [64][CUD]
-  // gridDim.x == ntiles: one tile per CTA (default); gridDim.x < ntiles (VGG_CHOL_PERSIST=1): a persistent CTA per SM walks
-  // the tiles, so that never more than one update CTA sits on an SM and a panel CTA of the next step always finds room.
-  // Measured r02: 0.920 ms against 0.890 -- one update CTA per SM hides its own latencies worse than it helps the panels.
-  for (int tile_t = blockIdx.x; tile_t < ntiles; tile_t += gridDim.x) {
   int bi, bj;
   {
-    int t = tile_t;
-    if (TM == 32) {
-      const int T = (n - t0 + 31) / 32;           // 32-row tiles; tile column 1 starts at row tile 2
-      if (t < T) { bi = t; bj = 0; }
-      else { bi = t - T + 2; bj = 1; }
-    } else if (mode == 4) {                         // tile columns 2 and 3 only (= block column k+2)
+    const int t = blockIdx.x;
+    if (mode == 4) {                         // tile columns 2 and 3 only (= block column k+2)
       const int T = (max(0, min(band_end, n) - t0) + 63) / 64 + (band_end >= n ? 0 : (n - arrow_lo + 63) / 64);
       if (t < T - 2) { bi = 2 + t; bj = 2; }
       else { bi = 3 + (t - (T - 2)); bj = 3; }
@@ -663,18 +607,18 @@ __global__ void __launch_bounds__(C_THREADS, 2) chol_update_kernel(int n, int ld
       while ((bi + 1) * (bi + 2) / 2 <= t) ++bi;
       while (bi * (bi + 1) / 2 > t) --bi;
       bj = t - bi * (bi + 1) / 2;
-      const int skip = mode == 5 ? 4 : (mode >= 2 ? 2 : 0);
+      const int skip = mode == 5 ? 4 : 0;
       bi += skip;
       bj += skip;
     }
   }
-  const bool diag = TM == 64 && bi == bj;
+  const bool diag = bi == bj;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   // banded matrices: 64-row tile v of the ACTIVE rows -- the band part [t0, band_end) first, then the arrow part
   // [arrow_lo, n) (band_end = n: the plain dense mapping)
   const int T1v = band_end >= n ? (1 << 30) : (band_end - t0) / 64;
   auto vrow = [&](int v) { return v < T1v ? t0 + v * 64 : arrow_lo + (v - T1v) * 64; };
-  const int ri = TM == 64 ? vrow(bi) : t0 + bi * TM, rj = TM == 64 ? vrow(bj) : t0 + bj * 64;
+  const int ri = vrow(bi), rj = vrow(bj);
   const double* bs = diag ? As : Bs;
   const int wm = warp / WN, wn = warp % WN;
   const int g = lane >> 2, q = lane & 3;
@@ -729,7 +673,7 @@ __global__ void __launch_bounds__(C_THREADS, 2) chol_update_kernel(int n, int ld
       const int col = rj + wn * (8 * NJ) + j * 8 + 2 * q;
       if (col > r) continue;                         // lower triangle only (col <= r < n)
       double* p = A + (size_t)r * lda + col;
-      if (TM == 64 && (all_red || (mode == 3 && bj < 4) || mode == 4 || (mode == 5 && bj < 6))) {
+      if (all_red || mode == 4 || (mode == 5 && bj < 6)) {
         atomicAdd(p, -c[i][j][0]);
         if (col + 1 <= r) atomicAdd(p + 1, -c[i][j][1]);
       } else if (col + 1 <= r) {
@@ -741,8 +685,6 @@ __global__ void __launch_bounds__(C_THREADS, 2) chol_update_kernel(int n, int ld
         *p -= c[i][j][0];
       }
     }
-  }
-  __syncthreads();                                  // the next tile's loads overwrite the operand buffers
   }
 }
 
@@ -757,8 +699,8 @@ size_t chol_workspace_doubles(int n) {
 namespace {
 
 struct CholStreams {
-  cudaStream_t side = nullptr, side_lo = nullptr, side_mid = nullptr, cap = nullptr;
-  cudaEvent_t ev_col = nullptr, ev_panel = nullptr, ev_upd[2] = {nullptr, nullptr}, ev_bulk[3] = {nullptr, nullptr, nullptr};
+  cudaStream_t side_lo = nullptr, side_mid = nullptr, cap = nullptr;
+  cudaEvent_t ev_col = nullptr, ev_upd[2] = {nullptr, nullptr}, ev_bulk[3] = {nullptr, nullptr, nullptr};
   bool ready = false;
 };
 
@@ -770,12 +712,10 @@ int chol_streams(CholStreams** out) {
     // lo = least, hi = greatest priority.  The critical chain (panel steps) is captured on `cap` at the greatest
     // priority; the fused schedule's bulk updates go to side_lo at the least, so that a panel CTA is placed as soon as
     // an SM has room for it instead of queueing behind the remaining update CTAs.
-    VGG_CUDA_CHECK(cudaStreamCreateWithPriority(&s.side, cudaStreamNonBlocking, hi));
     VGG_CUDA_CHECK(cudaStreamCreateWithPriority(&s.side_lo, cudaStreamNonBlocking, lo));
     VGG_CUDA_CHECK(cudaStreamCreateWithPriority(&s.side_mid, cudaStreamNonBlocking, (lo + hi) / 2));
     VGG_CUDA_CHECK(cudaStreamCreateWithPriority(&s.cap, cudaStreamNonBlocking, hi));
     VGG_CUDA_CHECK(cudaEventCreateWithFlags(&s.ev_col, cudaEventDisableTiming));
-    VGG_CUDA_CHECK(cudaEventCreateWithFlags(&s.ev_panel, cudaEventDisableTiming));
     VGG_CUDA_CHECK(cudaEventCreateWithFlags(&s.ev_upd[0], cudaEventDisableTiming));
     VGG_CUDA_CHECK(cudaEventCreateWithFlags(&s.ev_upd[1], cudaEventDisableTiming));
     for (int i = 0; i < 3; ++i) VGG_CUDA_CHECK(cudaEventCreateWithFlags(&s.ev_bulk[i], cudaEventDisableTiming));
@@ -785,23 +725,13 @@ int chol_streams(CholStreams** out) {
   return VGG_OK;
 }
 
-// VGG_CHOL_LEAF=0|1 (A/B): 8x8 leaf with one / two (default) pivots per step
-int chol_leaf() {
-  static const int v = [] { const char* e = getenv("VGG_CHOL_LEAF"); return (e && e[0] == '0') ? 0 : 1; }();
-  return v;
-}
-
 int chol_set_attrs() {
   static bool done = false;
   if (done) return VGG_OK;
-  VGG_CUDA_CHECK(cudaFuncSetAttribute(chol_panel_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+  VGG_CUDA_CHECK(cudaFuncSetAttribute(chol_panel_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       (int)(sizeof(double) * (CB + C_RPC) * CLD)));
-  VGG_CUDA_CHECK(cudaFuncSetAttribute(chol_panel_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      (int)(sizeof(double) * (CB + C_RPC) * CLD)));
-  VGG_CUDA_CHECK(cudaFuncSetAttribute(chol_update_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+  VGG_CUDA_CHECK(cudaFuncSetAttribute(chol_update_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       (int)(sizeof(double) * 2 * CT * CUD)));
-  VGG_CUDA_CHECK(cudaFuncSetAttribute(chol_update_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      (int)(sizeof(double) * (32 + CT) * CUD)));
   done = true;
   return VGG_OK;
 }
@@ -817,36 +747,17 @@ int g_chol_arrow_blk = 0;
 
 namespace {
 
-// VGG_CHOL_FUSE=0 (A/B): the r02 schedule with a separate critical-path update kernel per panel
-bool chol_fuse() {
-  static const bool v = [] { const char* e = getenv("VGG_CHOL_FUSE"); return !(e && e[0] == '0'); }();
-  return v;
-}
-
-// The launch sequence on (st, side).
-//   fused (default): step(b) = panel b + its update of block column b+1, all on st back to back; the rest of panel b's
-//     trailing update (block columns >= b+2) runs on the side stream behind step(b) and has to be finished before
+// The launch sequence on st and the side streams.
+//   fused (nblk >= 3): step(b) = panel b + its update of block column b+1, all on st back to back; the rest of panel b's
+//     trailing update (block columns >= b+2) runs on the side streams behind step(b) and has to be finished before
 //     step(b+2) -- it shares block column b+2 with step(b+1)'s fused update, both sides use REDs there.
-//   unfused lookahead: update<32>(b) [critical tiles] -> panel(b+1) on the side stream, update<64>(b) on st.
-//   lookahead == false: everything on st in program order.
-int chol_enqueue(int n, int lda, double* A, double* Ldiag, int* info, int* flags, cudaStream_t st, CholStreams* cs,
-                 bool lookahead) {
+//   program order (nblk < 3): update(b) then panel(b+1), everything on st; the matrix is treated as dense.
+int chol_enqueue(int n, int lda, double* A, double* Ldiag, int* info, int* flags, cudaStream_t st, CholStreams* cs) {
   const int nblk = (n + CB - 1) / CB;
   const size_t smem_p = sizeof(double) * (CB + C_RPC) * CLD;
   const size_t smem_u = sizeof(double) * 2 * CT * CUD;
-  const bool fuse = lookahead && chol_fuse();
-  static const int persist_ctas = [] {
-    const char* e = getenv("VGG_CHOL_PERSIST");
-    if (!(e && e[0] == '1')) return 0;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    return sms;
-  }();
-  auto upd_grid = [&](int tiles) { return persist_ctas > 0 ? std::min(tiles, persist_ctas) : tiles; };
-  static const bool split = [] { const char* e = getenv("VGG_CHOL_SPLIT"); return !(e && e[0] == '0'); }();
-  // the band structure is honoured by the default (fused + split) schedule only; the A/B schedules treat the matrix as dense
-  const bool banded = fuse && split && (int)g_chol_band_end.size() >= nblk && g_chol_arrow_blk > 0;
+  const bool fuse = nblk >= 3;
+  const bool banded = fuse && (int)g_chol_band_end.size() >= nblk && g_chol_arrow_blk > 0;
   auto band_rows = [&](int b, int* band_end, int* arrow_lo) {
     if (!banded) {
       *band_end = *arrow_lo = n;
@@ -856,28 +767,24 @@ int chol_enqueue(int n, int lda, double* A, double* Ldiag, int* info, int* flags
     *arrow_lo = std::min(n, std::max(g_chol_arrow_blk * CB, *band_end));
     if (*band_end >= n || *arrow_lo <= *band_end) *band_end = *arrow_lo = n;      // no gap left: plain dense rows
   };
-  auto panel = [&](int b, cudaStream_t s2) -> int {
+  auto panel = [&](int b) -> int {
     const int k0 = b * CB;
     int band_end, arrow_lo;
     band_rows(b, &band_end, &arrow_lo);
     const int below1 = std::max(0, std::min(band_end, n) - (k0 + CB));
     const int below2 = band_end >= n ? 0 : n - arrow_lo;
     const int chunks = (below1 + C_RPC - 1) / C_RPC + (below2 + C_RPC - 1) / C_RPC;
-    if (chol_leaf() == 1)
-      chol_panel_kernel<1><<<1 + chunks, C_THREADS, smem_p, s2>>>(n, lda, k0, A, Ldiag, info, flags, fuse ? 1 : 0, band_end, arrow_lo);
-    else
-      chol_panel_kernel<0><<<1 + chunks, C_THREADS, smem_p, s2>>>(n, lda, k0, A, Ldiag, info, flags, fuse ? 1 : 0, band_end, arrow_lo);
+    chol_panel_kernel<<<1 + chunks, C_THREADS, smem_p, st>>>(n, lda, k0, A, Ldiag, info, flags, fuse ? 1 : 0, band_end, arrow_lo);
     VGG_LAUNCH_CHECK();
     return VGG_OK;
   };
   int rc;
-  if ((rc = panel(0, st))) return rc;
+  if ((rc = panel(0))) return rc;
   if (fuse) {
     // Panel b's trailing update in two pieces with different deadlines: U1(b) = block column b+2 (needed by step(b+2),
     // one step of slack, medium priority) and U2(b) = block columns >= b+3 (needed by step(b+3), two steps of slack,
     // lowest priority).  r02: as ONE kernel with one step of slack the update of the first six panels did not fit
     // next to the following step and 0.15 ms of it showed up on the critical path.
-    static const bool skip_bulk = getenv("VGG_CHOL_TIMING_SKIP_BULK") != nullptr;   // timing experiment only: WRONG factor
     bool have_u1[2] = {false, false}, have_u2[3] = {false, false, false};
     for (int b = 0; b + 1 < nblk; ++b) {
       const int k0 = b * CB, t0 = k0 + CB;
@@ -887,38 +794,29 @@ int chol_enqueue(int n, int lda, double* A, double* Ldiag, int* info, int* flags
       const int all_red = band_end >= n ? 0 : 1;     // banded: tile columns no longer map to consecutive block columns
       const int n_u1 = T > 2 ? (T - 2) + (T > 3 ? T - 3 : 0) : 0;
       const int n_u2 = T > 4 ? (T - 4) * (T - 3) / 2 : 0;
-      const int n_rest = T > 2 ? (T - 2) * (T - 1) / 2 : 0;
       have_u1[b & 1] = false;
       have_u2[b % 3] = false;
-      if (n_rest > 0 && !skip_bulk) {
+      if (n_u1 > 0) {
         VGG_CUDA_CHECK(cudaEventRecord(cs->ev_col, st));                 // step(b) done
-        if (split) {
-          VGG_CUDA_CHECK(cudaStreamWaitEvent(cs->side_mid, cs->ev_col, 0));
-          // U2(b-2) still writes block column b+2 with plain read-modify-writes (only its first block column uses REDs)
-          if (b >= 2 && have_u2[(b - 2) % 3]) VGG_CUDA_CHECK(cudaStreamWaitEvent(cs->side_mid, cs->ev_bulk[(b - 2) % 3], 0));
-          chol_update_kernel<64><<<upd_grid(n_u1), C_THREADS, smem_u, cs->side_mid>>>(n, lda, k0, t0, 4, A, band_end, arrow_lo, all_red, n_u1);
-          VGG_LAUNCH_CHECK();
-          VGG_CUDA_CHECK(cudaEventRecord(cs->ev_upd[b & 1], cs->side_mid));
-          have_u1[b & 1] = true;
-          if (n_u2 > 0) {
-            VGG_CUDA_CHECK(cudaStreamWaitEvent(cs->side_lo, cs->ev_col, 0));
-            chol_update_kernel<64><<<upd_grid(n_u2), C_THREADS, smem_u, cs->side_lo>>>(n, lda, k0, t0, 5, A, band_end, arrow_lo, all_red, n_u2);
-            VGG_LAUNCH_CHECK();
-            VGG_CUDA_CHECK(cudaEventRecord(cs->ev_bulk[b % 3], cs->side_lo));
-            have_u2[b % 3] = true;
-          }
-        } else {
+        VGG_CUDA_CHECK(cudaStreamWaitEvent(cs->side_mid, cs->ev_col, 0));
+        // U2(b-2) still writes block column b+2 with plain read-modify-writes (only its first block column uses REDs)
+        if (b >= 2 && have_u2[(b - 2) % 3]) VGG_CUDA_CHECK(cudaStreamWaitEvent(cs->side_mid, cs->ev_bulk[(b - 2) % 3], 0));
+        chol_update_kernel<<<n_u1, C_THREADS, smem_u, cs->side_mid>>>(n, lda, k0, t0, 4, A, band_end, arrow_lo, all_red);
+        VGG_LAUNCH_CHECK();
+        VGG_CUDA_CHECK(cudaEventRecord(cs->ev_upd[b & 1], cs->side_mid));
+        have_u1[b & 1] = true;
+        if (n_u2 > 0) {
           VGG_CUDA_CHECK(cudaStreamWaitEvent(cs->side_lo, cs->ev_col, 0));
-          chol_update_kernel<64><<<upd_grid(n_rest), C_THREADS, smem_u, cs->side_lo>>>(n, lda, k0, t0, 3, A, n, n, 0, n_rest);
+          chol_update_kernel<<<n_u2, C_THREADS, smem_u, cs->side_lo>>>(n, lda, k0, t0, 5, A, band_end, arrow_lo, all_red);
           VGG_LAUNCH_CHECK();
-          VGG_CUDA_CHECK(cudaEventRecord(cs->ev_upd[b & 1], cs->side_lo));
-          have_u1[b & 1] = true;
+          VGG_CUDA_CHECK(cudaEventRecord(cs->ev_bulk[b % 3], cs->side_lo));
+          have_u2[b % 3] = true;
         }
       }
       // step(b+1) factors block column b+1: U1(b-1) (the last update of panel b-1 that touches it) and U2(b-2) must be done
       if (b >= 1 && have_u1[(b - 1) & 1]) VGG_CUDA_CHECK(cudaStreamWaitEvent(st, cs->ev_upd[(b - 1) & 1], 0));
       if (b >= 2 && have_u2[(b - 2) % 3]) VGG_CUDA_CHECK(cudaStreamWaitEvent(st, cs->ev_bulk[(b - 2) % 3], 0));
-      if ((rc = panel(b + 1, st))) return rc;
+      if ((rc = panel(b + 1))) return rc;
     }
     // join whatever the last two panels left on the side streams (capture needs every forked stream back)
     for (int i = 0; i < 2; ++i)
@@ -930,26 +828,9 @@ int chol_enqueue(int n, int lda, double* A, double* Ldiag, int* info, int* flags
   for (int b = 0; b + 1 < nblk; ++b) {
     const int k0 = b * CB, t0 = k0 + CB;
     const int T = (n - t0 + CT - 1) / CT;
-    const int T32 = (n - t0 + 31) / 32;
-    const int n_col = T32 + (T32 > 2 ? T32 - 2 : 0);       // 32-row tiles of tile columns 0 and 1
-    const int n_rest = T > 2 ? (T - 2) * (T - 1) / 2 : 0;
-    if (!lookahead) {
-      chol_update_kernel<64><<<upd_grid(T * (T + 1) / 2), C_THREADS, smem_u, st>>>(n, lda, k0, t0, 0, A, n, n, 0, T * (T + 1) / 2);
-      VGG_LAUNCH_CHECK();
-      if ((rc = panel(b + 1, st))) return rc;
-      continue;
-    }
-    chol_update_kernel<32><<<n_col, C_THREADS, sizeof(double) * (32 + CT) * CUD, st>>>(n, lda, k0, t0, 1, A, n, n, 0, n_col);
+    chol_update_kernel<<<T * (T + 1) / 2, C_THREADS, smem_u, st>>>(n, lda, k0, t0, 0, A, n, n, 0);
     VGG_LAUNCH_CHECK();
-    VGG_CUDA_CHECK(cudaEventRecord(cs->ev_col, st));
-    VGG_CUDA_CHECK(cudaStreamWaitEvent(cs->side, cs->ev_col, 0));
-    if ((rc = panel(b + 1, cs->side))) return rc;
-    VGG_CUDA_CHECK(cudaEventRecord(cs->ev_panel, cs->side));
-    if (n_rest > 0) {
-      chol_update_kernel<64><<<upd_grid(n_rest), C_THREADS, smem_u, st>>>(n, lda, k0, t0, 2, A, n, n, 0, n_rest);
-      VGG_LAUNCH_CHECK();
-    }
-    VGG_CUDA_CHECK(cudaStreamWaitEvent(st, cs->ev_panel, 0));
+    if ((rc = panel(b + 1))) return rc;
   }
   return VGG_OK;
 }
@@ -958,7 +839,7 @@ int chol_enqueue(int n, int lda, double* A, double* Ldiag, int* info, int* flags
 
 // In-place Cholesky of the row-major lower triangle of A[n x n] (lda even, A 16-byte aligned): on return the lower
 // triangle holds L and the strict upper triangle L^T.  info (device int): 0 or the 1-based index of the first
-// non-positive pivot.  VGG_CHOL_LOOKAHEAD=0 / VGG_CHOL_GRAPH=0 switch the side stream / the CUDA graph off (A/B).
+// non-positive pivot.
 int chol_lower_inplace(int n, int lda, double* A, double* Ldiag, int* info, cudaStream_t st) {
   VGG_REQUIRE((lda % 2) == 0, "lda must be even");
   int rc;
@@ -967,24 +848,22 @@ int chol_lower_inplace(int n, int lda, double* A, double* Ldiag, int* info, cuda
   const int nblk0 = (n + CB - 1) / CB;
   int* flags = reinterpret_cast<int*>(Ldiag + (size_t)nblk0 * CB * CB);
   VGG_CUDA_CHECK(cudaMemsetAsync(flags, 0, sizeof(int) * (size_t)nblk0, st));
-  static const bool lookahead = [] { const char* e = getenv("VGG_CHOL_LOOKAHEAD"); return !(e && e[0] == '0'); }();
-  static const bool use_graph = [] { const char* e = getenv("VGG_CHOL_GRAPH"); return !(e && e[0] == '0'); }();
   const int nblk = (n + CB - 1) / CB;
   CholStreams* cs = nullptr;
   if ((rc = chol_streams(&cs))) return rc;
-  if (nblk < 3 || !use_graph) return chol_enqueue(n, lda, A, Ldiag, info, flags, st, cs, lookahead && nblk >= 3);
+  if (nblk < 3) return chol_enqueue(n, lda, A, Ldiag, info, flags, st, cs);
   // one captured graph per (matrix, order): ~60 launches + events become a single cudaGraphLaunch
-  typedef std::tuple<double*, int, int, int*, double*, bool, unsigned long long> Key;
+  typedef std::tuple<double*, int, int, int*, double*, unsigned long long> Key;
   static thread_local std::map<Key, cudaGraphExec_t> cache;
   unsigned long long band_hash = (unsigned long long)g_chol_arrow_blk;
   for (int v : g_chol_band_end) band_hash = band_hash * 1000003ull + (unsigned long long)(v + 1);
-  const Key key(A, n, lda, info, Ldiag, lookahead, band_hash);
+  const Key key(A, n, lda, info, Ldiag, band_hash);
   auto it = cache.find(key);
   if (it == cache.end()) {
     const long long launches_before = g_launch_count;
     cudaGraph_t graph = nullptr;
     VGG_CUDA_CHECK(cudaStreamBeginCapture(cs->cap, cudaStreamCaptureModeThreadLocal));
-    rc = chol_enqueue(n, lda, A, Ldiag, info, flags, cs->cap, cs, lookahead);
+    rc = chol_enqueue(n, lda, A, Ldiag, info, flags, cs->cap, cs);
     const cudaError_t ce = cudaStreamEndCapture(cs->cap, &graph);
     g_launch_count = launches_before;
     if (rc) {
@@ -1009,7 +888,7 @@ int chol_lower_inplace(int n, int lda, double* A, double* Ldiag, int* info, cuda
 }  // namespace vgg
 
 // tools/microbench.py chol128: one CTA, POTRF128 of A (host, row-major SPD 128 x 128), cycles per phase
-extern "C" int vgg_dev_chol128_probe(int leaf, int reps, const double* A_host, double* L_host, long long* prof13_host) {
+extern "C" int vgg_dev_chol128_probe(int reps, const double* A_host, double* L_host, long long* prof13_host) {
   using namespace vgg;
   VGG_REQUIRE(A_host && L_host && prof13_host && reps > 0, "chol128 probe: bad arguments");
   double *dA = nullptr, *dL = nullptr;
@@ -1020,13 +899,8 @@ extern "C" int vgg_dev_chol128_probe(int leaf, int reps, const double* A_host, d
   VGG_CUDA_CHECK(cudaMemcpy(dA, A_host, sizeof(double) * CB * CB, cudaMemcpyHostToDevice));
   VGG_CUDA_CHECK(cudaMemset(dP, 0, sizeof(long long) * 13));
   const int smem = (int)(sizeof(double) * (CB + C_RPC) * CLD);
-  if (leaf == 1) {
-    VGG_CUDA_CHECK(cudaFuncSetAttribute(chol128_probe_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    chol128_probe_kernel<1><<<1, C_THREADS, smem>>>(dA, dL, dP, reps, C_RPC);
-  } else {
-    VGG_CUDA_CHECK(cudaFuncSetAttribute(chol128_probe_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    chol128_probe_kernel<0><<<1, C_THREADS, smem>>>(dA, dL, dP, reps, C_RPC);
-  }
+  VGG_CUDA_CHECK(cudaFuncSetAttribute(chol128_probe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  chol128_probe_kernel<<<1, C_THREADS, smem>>>(dA, dL, dP, reps, C_RPC);
   VGG_LAUNCH_CHECK();
   VGG_CUDA_CHECK(cudaDeviceSynchronize());
   VGG_CUDA_CHECK(cudaMemcpy(L_host, dL, sizeof(double) * CB * CB, cudaMemcpyDeviceToHost));

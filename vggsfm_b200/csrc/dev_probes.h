@@ -8,18 +8,16 @@ extern "C" {
  * bit0 selects N=256 (else 128), mode>>1 the shared-memory layout (0 = 64 B swizzle, 1 = 128 B swizzle, 2 = none).
  * out_cycles is a host pointer. */
 int vgg_syrk_ozaki_mma_rate(int iters, int mode, double* out_cycles, void* stream);
-/* Cluster hardware-rule probe used while developing the CTA-pair SYRK (bounded, cannot hang): out_host[0..2] int. */
-int vgg_probe_remote_mbarrier(int* out_host, void* stream);
 /* Kernel-only timing of ba_blocks_kernel: while enabled, every build_blocks call records a CUDA event pair on its stream
  * directly around the kernel launch (the accumulator memsets before it are outside); last_ms waits for the second event
  * and returns the elapsed milliseconds of the most recent launch. */
 int vgg_dev_blocks_timing(int enable);
 int vgg_dev_blocks_last_ms(double* ms);
-/* One-CTA probe of the in-shared-memory POTRF128 of csrc/chol.cu (leaf 0|1 = one / two pivots per 8x8 leaf step):
+/* One-CTA probe of the in-shared-memory POTRF128 of csrc/chol.cu:
  * A_host row-major SPD 128 x 128, L_host its factor, prof13_host[0..5] = cycles per phase seen by warp 0, [6..11] by
  * warp 1 (0 first leaf, 1 TRSM of the micro-panel, 2 look-ahead section work, 3 wait at its barrier, 4 rank-32 DMMA
  * update, 5 first leaf of the next sub-panel), [12] = total cycles of the last of `reps` passes. */
-int vgg_dev_chol128_probe(int leaf, int reps, const double* A_host, double* L_host, long long* prof13_host);
+int vgg_dev_chol128_probe(int reps, const double* A_host, double* L_host, long long* prof13_host);
 /* Band hint of the tensor-core SYRK for tests: ranges_host[2*rb], [2*rb+1] = the 64-row k-block range outside which the
  * 128-column row block rb of Zt is exactly zero (count = 2 * Dpad/128; count = 0 clears it).  vgg_ba_solve computes the
  * same thing from the visibility mask and clears it when it returns. */

@@ -10,7 +10,7 @@
 //      every C_t is an exact int32 (|d| <= 128, at most 7 pairs and 16384 k per work item: |C_t| < 2^31); orders t > s+1 are below
 //      the rounding of step 1 and are dropped, leaving s(s+1)/2 int8 GEMMs (28 for s = 7)  (oz_syrk_kernel)
 //   3. the epilogue recombines the C_t of a tile in FP64 registers and adds -value into Sraw with f64 RED
-//      (or multimem.red in fabric mode), exactly like the DMMA kernel's epilogue.
+//      (multimem.red or a remote RED in the multi-GPU modes).
 //
 // oz_syrk_kernel is a persistent, warp-specialised tcgen05 kernel (one CTA per SM):
 //   warp 0   producer: the int8 slices are stored in HBM as 8 KB tile images that are already in the 64-byte
@@ -20,7 +20,7 @@
 //            (p,q) pair of the work item's order group into up to four 128-column TMEM accumulators (one per order
 //            t), tcgen05.commit releases the smem stage / publishes the accumulators;
 //   warps 2-9 epilogue: tcgen05.ld the accumulators, combine the orders in FP64 registers, release TMEM, then
-//            scale by 2^(e_i+e_j) and RED into both triangles while the next item's MMAs already run.
+//            scale by 2^(e_i+e_j) and RED into the lower triangle while the next item's MMAs already run.
 // Work items (tile, order group, k range) are built on the host, longest first, and strided over the CTAs.
 #include "common.cuh"
 #include "dev_probes.h"
@@ -39,13 +39,11 @@ constexpr int OZ_STAGES = 2;
 constexpr int OZ_STAGE_TILES = 14;
 constexpr int OZ_STAGE_BYTES = OZ_STAGE_TILES * OZ_TILE_BYTES;   // 112 KB
 constexpr int OZ_THREADS = 320;                  // producer warp, MMA warp, 8 epilogue warps
-constexpr int OZ_THREADS_TS = 448;               // + 4 warps that stage the A operand in tensor memory (A-in-TMEM variant)
-constexpr int OZ_TS_ACOL = 384;                  // TMEM columns 384..495: two buffers x 7 slices x 8 columns (K = 32 int8)
-constexpr int OZ_TS_ABUF = 56;
 constexpr int OZ_MAX_PAIRS = 20;
 constexpr int OZ_MAX_ITEM_KB = 256;               // k blocks per work item: 7 pairs x 128^2 x 256 x 64 < 2^31 (exact int32 accumulators)
 constexpr int OZ_PREFETCH = 4;                   // k blocks of L2 prefetch distance ahead of the bulk copies
 constexpr int OZ_MAX_GROUPS = 3;
+constexpr int OZ_MAX_ACC = 4;                    // 128-column TMEM accumulators (orders) per group
 constexpr int OZ_EXPO_BAD = INT32_MIN;           // column holds a non-finite value
 constexpr size_t OZ_SMEM_BYTES = (size_t)OZ_STAGES * OZ_STAGE_BYTES + 1024 + 128;
 
@@ -173,7 +171,7 @@ __device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint64_t desc_a, uint64
       : "memory");
 }
 // same with the A operand in tensor memory (128 lanes = rows, 8 32-bit columns = 32 int8 of K per row): the MMA then
-// reads only B from shared memory
+// reads only B from shared memory (oz_mma_rate_kernel)
 __device__ __forceinline__ void umma_i8_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t desc_b, uint32_t idesc,
                                            uint32_t accumulate) {
   asm volatile(
@@ -205,14 +203,6 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
       : "r"(taddr));
   asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
-// 32 lanes x 8 columns: lane l of the warp writes its 32 bytes (one row of an int8 A operand, K = 32) into TMEM lane
-// (warp % 4) * 32 + l, columns taddr .. taddr + 7
-__device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint4& a, const uint4& b) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};\n" ::"r"(taddr), "r"(a.x), "r"(a.y),
-               "r"(a.z), "r"(a.w), "r"(b.x), "r"(b.y), "r"(b.z), "r"(b.w)
-               : "memory");
-}
-__device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 // shared-memory matrix descriptor: K-major, 64-byte swizzle, 8-row atoms 512 B apart, sm_100 descriptor version
 __device__ __forceinline__ uint64_t smem_desc_sw64(uint32_t saddr) {
   return (uint64_t)((saddr >> 4) & 0x3FFF) | ((uint64_t)(512 >> 4) << 32) | (1ull << 46) | (4ull << 61);
@@ -222,31 +212,21 @@ constexpr uint32_t OZ_IDESC = (2u << 4) | (1u << 7) | (1u << 10) | ((128u >> 3) 
 
 // ---------------------------------------------------------------------------------------------------------
 // 3. persistent tcgen05 SYRK
-// TS = true: A-in-TMEM variant.  r01 found the SS kernel bound by shared-memory bandwidth, not by the tensor pipe: every
-// N = 128 MMA re-reads its 4 KB A operand and its 4 KB B operand (28 pairs x 2 x 8 KB = 448 KB per 64-byte k-block, plus
-// the 112 KB the bulk copies write, at 128 B/clk = 4.4 k clk against 3.6 k clk of tensor work).  Here four extra warps
-// copy the <= 7 A slices of a k-block from shared memory into tensor memory once (tcgen05.st, 8 columns per slice and
-// K = 32 half, double buffered) and the MMAs take A from there: 224 KB of B reads + 56 KB of staging reads per k-block.
-// Tensor memory: three 128-column accumulators (order groups of <= 3) + 112 columns of A.
-// MEASURED (r02, 400 x 4096: Dpad 2432, K 12288): exact (6.6e-16, all parity tests pass with VGG_SYRK_TS=1) but SLOWER,
-// 1.86 ms per call against 1.07 ms: with tensor memory full there is room for two K = 32 halves of A only, so every
-// half pays a staging round (wait for the MMAs two halves back, 7 x (2 LDS.128 + tcgen05.st), wait::st, fence, barrier)
-// that is longer than the ~15 MMAs it feeds.  Kept behind VGG_SYRK_TS=1 as a record; the default stays the SS kernel.
-template <bool TS>
-__global__ void __maxnreg__(TS ? 128 : 168)      // 448 x 128 / 320 x 168 registers (448 x 144 does not launch: "too many resources")
+// Two variants were measured slower on a B200 and removed (profiles/README.md): the A operand staged in tensor memory by
+// four extra warps (exact, 1.86 ms per call against 1.07 ms at 400 x 4096: the staging round per K = 32 half outlasts the
+// ~15 MMAs it feeds) and CTA pairs issuing cta_group::2 MMAs with M = 256 (exact, 1.21 ms against 1.07 ms).
+__global__ void __maxnreg__(168)                 // 320 threads x 168 registers
     oz_syrk_kernel(const __grid_constant__ OzPlan plan, const OzWork* __restrict__ work, int nwork, int KB,
                    const int8_t* __restrict__ slices, size_t slice_stride, const int* __restrict__ expo,
                    const double* __restrict__ pow2, int Dpad, double* __restrict__ Cmat, ptrdiff_t mc_off,
-                   int fill_upper, const __grid_constant__ FabricDev fd) {
+                   const __grid_constant__ FabricDev fd) {
   extern __shared__ __align__(1024) uint8_t oz_smem[];
   uint8_t* tiles = reinterpret_cast<uint8_t*>(align_up(reinterpret_cast<size_t>(oz_smem), 1024));
   uint64_t* full = reinterpret_cast<uint64_t*>(tiles + (size_t)OZ_STAGES * OZ_STAGE_BYTES);
   uint64_t* empty = full + OZ_STAGES;
   uint64_t* tmem_full = empty + OZ_STAGES;
   uint64_t* tmem_empty = tmem_full + 1;
-  uint64_t* a_full = tmem_empty + 1;             // [2] (TS): A buffer staged in tensor memory, one arrive per staging warp
-  uint64_t* a_empty = a_full + 2;                // [2] (TS): the MMAs that read the buffer have completed
-  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(a_empty + 2);
+  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(tmem_empty + 1);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
   if (threadIdx.x == 0) {
@@ -256,10 +236,6 @@ __global__ void __maxnreg__(TS ? 128 : 168)      // 448 x 128 / 320 x 168 regist
     }
     mbar_init(tmem_full, 1);
     mbar_init(tmem_empty, 8);
-    for (int s = 0; s < 2; ++s) {
-      mbar_init(&a_full[s], 4);
-      mbar_init(&a_empty[s], 1);
-    }
     mbar_fence_init();
   }
   if (warp == 1) tmem_alloc(tmem_ptr, 512);
@@ -306,9 +282,6 @@ __global__ void __maxnreg__(TS ? 128 : 168)      // 448 x 128 / 320 x 168 regist
     // ===== MMA issuer =====
     if (lane == 0) {
       int stage = 0, phase = 0, it = 0;
-      int abuf = 0, aphase = 0;
-      (void)abuf;
-      (void)aphase;
       for (int w = blockIdx.x; w < nwork; w += gridDim.x, ++it) {
         const OzWork wk = work[w];
         const OzGroup& g = plan.g[wk.group];
@@ -320,32 +293,15 @@ __global__ void __maxnreg__(TS ? 128 : 168)      // 448 x 128 / 320 x 168 regist
           mbar_wait(&full[stage], phase);
           tc_fence_after();
           const uint32_t base = smem_u32(tiles + (size_t)stage * OZ_STAGE_BYTES);
-          if (TS) {
-            for (int ks = 0; ks < OZ_BK / 32; ++ks) {
-              mbar_wait(&a_full[abuf], aphase);
-              tc_fence_after();
-              const uint32_t a_base = tmem_base + (uint32_t)(OZ_TS_ACOL + abuf * OZ_TS_ABUF);
-              for (int pr = 0; pr < g.n_pairs; ++pr) {
-                const uint32_t b_addr = base + (uint32_t)(diag ? g.pair_b_diag[pr] : g.n_a + g.pair_b[pr]) * OZ_TILE_BYTES;
-                const uint32_t acc = g.pair_acc[pr];
-                umma_i8_ts(tmem_base + acc * 128u, a_base + (uint32_t)g.pair_a[pr] * 8u, smem_desc_sw64(b_addr + ks * 32),
-                           OZ_IDESC, (acc_used >> acc) & 1u);
-                acc_used |= 1u << acc;
-              }
-              umma_commit(&a_empty[abuf]);
-              if ((abuf ^= 1) == 0) aphase ^= 1;
-            }
-          } else {
-            for (int pr = 0; pr < g.n_pairs; ++pr) {
-              const uint32_t a_addr = base + (uint32_t)g.pair_a[pr] * OZ_TILE_BYTES;
-              const uint32_t b_addr = base + (uint32_t)(diag ? g.pair_b_diag[pr] : g.n_a + g.pair_b[pr]) * OZ_TILE_BYTES;
-              const uint32_t acc = g.pair_acc[pr];
+          for (int pr = 0; pr < g.n_pairs; ++pr) {
+            const uint32_t a_addr = base + (uint32_t)g.pair_a[pr] * OZ_TILE_BYTES;
+            const uint32_t b_addr = base + (uint32_t)(diag ? g.pair_b_diag[pr] : g.n_a + g.pair_b[pr]) * OZ_TILE_BYTES;
+            const uint32_t acc = g.pair_acc[pr];
 #pragma unroll
-              for (int ks = 0; ks < OZ_BK / 32; ++ks) {
-                umma_i8(tmem_base + acc * 128u, smem_desc_sw64(a_addr + ks * 32), smem_desc_sw64(b_addr + ks * 32),
-                        OZ_IDESC, (acc_used >> acc) & 1u);
-                acc_used |= 1u << acc;
-              }
+            for (int ks = 0; ks < OZ_BK / 32; ++ks) {
+              umma_i8(tmem_base + acc * 128u, smem_desc_sw64(a_addr + ks * 32), smem_desc_sw64(b_addr + ks * 32),
+                      OZ_IDESC, (acc_used >> acc) & 1u);
+              acc_used |= 1u << acc;
             }
           }
           umma_commit(&empty[stage]);
@@ -355,40 +311,6 @@ __global__ void __maxnreg__(TS ? 128 : 168)      // 448 x 128 / 320 x 168 regist
           }
         }
         umma_commit(tmem_full);
-      }
-    }
-  } else if (TS && warp >= 10) {
-    // ===== A staging (4 warps, TMEM lane quarter = warp % 4): shared memory -> tensor memory, one K = 32 half at a time =====
-    const int quarter = warp & 3;
-    const int row = quarter * 32 + lane;
-    const uint32_t sw = (uint32_t)((row >> 1) & 3);
-    int stage = 0, phase = 0, abuf = 0, aphase = 0;
-    for (int w = blockIdx.x; w < nwork; w += gridDim.x) {
-      const OzWork wk = work[w];
-      const OzGroup& g = plan.g[wk.group];
-      for (int kb = wk.kb0; kb < wk.kb1; ++kb) {
-        mbar_wait(&full[stage], phase);                       // this k-block's tile images have landed
-        const uint8_t* st_tiles = tiles + (size_t)stage * OZ_STAGE_BYTES + (size_t)row * OZ_BK;
-        for (int ks = 0; ks < OZ_BK / 32; ++ks) {
-          mbar_wait(&a_empty[abuf], (uint32_t)(aphase ^ 1));  // the MMAs that read this buffer two halves ago are done
-          tc_fence_after();
-          const uint32_t t_base = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(OZ_TS_ACOL + abuf * OZ_TS_ABUF);
-          for (int i = 0; i < g.n_a; ++i) {
-            const uint8_t* trow = st_tiles + (size_t)i * OZ_TILE_BYTES;
-            const uint4 v0 = *reinterpret_cast<const uint4*>(trow + ((((uint32_t)(2 * ks)) ^ sw) << 4));
-            const uint4 v1 = *reinterpret_cast<const uint4*>(trow + ((((uint32_t)(2 * ks + 1)) ^ sw) << 4));
-            tmem_st8(t_base + (uint32_t)i * 8u, v0, v1);
-          }
-          tmem_wait_st();
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&a_full[abuf]);
-          if ((abuf ^= 1) == 0) aphase ^= 1;
-        }
-        if (++stage == OZ_STAGES) {
-          stage = 0;
-          phase ^= 1;
-        }
       }
     }
   } else {
@@ -417,7 +339,7 @@ __global__ void __maxnreg__(TS ? 128 : 168)      // 448 x 128 / 320 x 168 regist
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(tmem_empty);
-      // scale and accumulate into Sraw (same triangle rules as syrk_dmma_kernel)
+      // scale and accumulate into Sraw
       const int r = wk.bi * OZ_BM + row_local;
       const int er = expo[r];
       const bool diag = wk.bi == wk.bj;
@@ -435,8 +357,7 @@ __global__ void __maxnreg__(TS ? 128 : 168)      // 448 x 128 / 320 x 168 regist
         if (v != 0.0) {
           // The work list holds UPPER tiles (bi <= bj): TMEM lane = r, so the 32 lanes of one RED instruction hit 32
           // consecutive addresses of row `col` -- the mirrored element (col, r) of the row-major LOWER triangle, which is
-          // what csrc/chol.cu factors (fabric mode: one multimem op per element).  The direct element (r, col) is only
-          // written for the library factorisation A/B.
+          // what csrc/chol.cu factors (fabric mode: one multimem op per element).
           if (!diag || col >= r) {
             const size_t off = (size_t)col * Dpad + r;
             if (fd.world > 1) {
@@ -449,7 +370,6 @@ __global__ void __maxnreg__(TS ? 128 : 168)      // 448 x 128 / 320 x 168 regist
               atomicAdd(Cmat + off, -v);
             }
           }
-          if (fill_upper && (!diag || col > r)) atomicAdd(&Cmat[(size_t)r * Dpad + col], -v);
         }
       }
     }
@@ -459,316 +379,6 @@ __global__ void __maxnreg__(TS ? 128 : 168)      // 448 x 128 / 320 x 168 regist
   if (warp == 1) tmem_dealloc(tmem_base, 512);
 }
 
-
-
-// ---------------------------------------------------------------------------------------------------------
-// 3b. CTA-pair variant (VGG_SYRK_PAIR=1): a cluster of two CTAs owns two row blocks (bi0, bi1) of one column block bj and
-// issues tcgen05.mma.cta_group::2 (M = 256 = 128 rows per CTA, N = 128, K = 32).  Each CTA stages its own A tiles and
-// only HALF of every B tile (64 of the 128 rows: the first / second 4 KB of the pre-swizzled tile image), so per-CTA
-// shared-memory and L2->SM traffic drop by a quarter and the MMA issues at the full-rate M=256 shape.
-//   * loads: every CTA's producer fills its own stage and its own full barrier; the peer's warp 1 relays "my stage is
-//     full" to the leader with a remote mbarrier arrive (a 1-D bulk copy cannot signal another CTA's barrier);
-//   * MMAs are issued by the leader only; tcgen05.commit multicasts the arrival to both CTAs' empty / tmem_full barriers;
-//   * both epilogues read their own TMEM (their 128 rows) and arrive on the leader's tmem_empty barrier.
-struct OzWork2 {
-  int bi0, bi1, bj, group, kb0, kb1, dup;       // dup: bi1 repeats bi0 (odd tile count in a column); CTA 1 discards
-};
-constexpr int OZ2_STAGE_BYTES = 7 * OZ_TILE_BYTES + 7 * (OZ_TILE_BYTES / 2);   // 84 KB
-constexpr int OZ2_STAGES = 2;
-constexpr size_t OZ2_SMEM_BYTES = (size_t)OZ2_STAGES * OZ2_STAGE_BYTES + 1024 + 256;
-constexpr uint32_t OZ_IDESC2 = (2u << 4) | (1u << 7) | (1u << 10) | ((128u >> 3) << 17) | ((256u >> 4) << 24);
-
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t mapa_shared(uint32_t saddr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(saddr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "WAIT_LOOP_C:\n"
-      "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra DONE_C;\n"
-      "bra WAIT_LOOP_C;\n"
-      "DONE_C:\n"
-      "}\n" ::"r"(smem_u32(bar)),
-      "r"(parity)
-      : "memory");
-}
-__device__ __forceinline__ void tmem_alloc2(uint32_t* dst_smem, uint32_t cols) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(cols)
-               : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc2(uint32_t taddr, uint32_t cols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
-}
-__device__ __forceinline__ void umma_i8_2cta(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                             uint32_t accumulate) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "setp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::2.kind::i8 [%0], %1, %2, %3, p;\n"
-      "}\n" ::"r"(tmem_d),
-      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit_2cta(uint64_t* bar) {
-  asm volatile(
-      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-          smem_u32(bar)),
-      "h"((uint16_t)3)
-      : "memory");
-}
-
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(OZ_THREADS, 1)
-    oz_syrk_pair_kernel(const __grid_constant__ OzPlan plan, const OzWork2* __restrict__ work, int nwork, int KB,
-                        const int8_t* __restrict__ slices, size_t slice_stride, const int* __restrict__ expo,
-                        const double* __restrict__ pow2, int Dpad, double* __restrict__ Cmat, ptrdiff_t mc_off,
-                   int fill_upper) {
-  extern __shared__ __align__(1024) uint8_t oz_smem[];
-  uint8_t* tiles = reinterpret_cast<uint8_t*>(align_up(reinterpret_cast<size_t>(oz_smem), 1024));
-  uint64_t* full = reinterpret_cast<uint64_t*>(tiles + (size_t)OZ2_STAGES * OZ2_STAGE_BYTES);
-  uint64_t* empty = full + OZ2_STAGES;
-  uint64_t* peer_full = empty + OZ2_STAGES;      // leader only: "the peer's stage is full"
-  uint64_t* tmem_full = peer_full + OZ2_STAGES;
-  uint64_t* tmem_empty = tmem_full + 1;          // leader only: 16 epilogue warps of the pair
-  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(tmem_empty + 1);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  const int cluster_id = blockIdx.x >> 1, nclusters = gridDim.x >> 1;
-
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < OZ2_STAGES; ++s) {
-      mbar_init(&full[s], 1);
-      mbar_init(&empty[s], 1);
-      mbar_init(&peer_full[s], 1);
-    }
-    mbar_init(tmem_full, 1);
-    mbar_init(tmem_empty, 16);
-    mbar_fence_init();
-  }
-  if (warp == 1) tmem_alloc2(tmem_ptr, 512);
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr;
-
-  if (warp == 0) {
-    // ===== producer (both CTAs): own A tiles, own half of every B tile =====
-    if (lane == 0) {
-      int stage = 0, phase = 0;
-      for (int w = cluster_id; w < nwork; w += nclusters) {
-        const OzWork2 wk = work[w];
-        const OzGroup& g = plan.g[wk.group];
-        const int bi = rank ? wk.bi1 : wk.bi0;
-        for (int kb = wk.kb0; kb < wk.kb1; ++kb) {
-          mbar_wait(&empty[stage], phase ^ 1);
-          uint8_t* dst = tiles + (size_t)stage * OZ2_STAGE_BYTES;
-          mbar_expect_tx(&full[stage], (uint32_t)(g.n_a * OZ_TILE_BYTES + g.n_b * (OZ_TILE_BYTES / 2)));
-          for (int i = 0; i < g.n_a; ++i)
-            tma_load_1d(dst + (size_t)i * OZ_TILE_BYTES,
-                        slices + (size_t)g.a_slice[i] * slice_stride + ((size_t)bi * KB + kb) * OZ_TILE_BYTES, OZ_TILE_BYTES,
-                        &full[stage]);
-          for (int i = 0; i < g.n_b; ++i)
-            tma_load_1d(dst + (size_t)g.n_a * OZ_TILE_BYTES + (size_t)i * (OZ_TILE_BYTES / 2),
-                        slices + (size_t)g.b_slice[i] * slice_stride + ((size_t)wk.bj * KB + kb) * OZ_TILE_BYTES +
-                            (size_t)rank * (OZ_TILE_BYTES / 2),
-                        OZ_TILE_BYTES / 2, &full[stage]);
-          if (++stage == OZ2_STAGES) {
-            stage = 0;
-            phase ^= 1;
-          }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0) {
-      int stage = 0, phase = 0, it = 0;
-      if (rank == 0) {
-        // ===== MMA issuer (leader) =====
-        for (int w = cluster_id; w < nwork; w += nclusters, ++it) {
-          const OzWork2 wk = work[w];
-          const OzGroup& g = plan.g[wk.group];
-          mbar_wait_cluster(tmem_empty, (uint32_t)((it & 1) ^ 1));
-          tc_fence_after();
-          uint32_t acc_used = 0;
-          for (int kb = wk.kb0; kb < wk.kb1; ++kb) {
-            mbar_wait(&full[stage], phase);
-            mbar_wait_cluster(&peer_full[stage], phase);
-            tc_fence_after();
-            const uint32_t base = smem_u32(tiles + (size_t)stage * OZ2_STAGE_BYTES);
-            for (int pr = 0; pr < g.n_pairs; ++pr) {
-              const uint32_t a_addr = base + (uint32_t)g.pair_a[pr] * OZ_TILE_BYTES;
-              const uint32_t b_addr = base + (uint32_t)g.n_a * OZ_TILE_BYTES + (uint32_t)g.pair_b[pr] * (OZ_TILE_BYTES / 2);
-              const uint32_t acc = g.pair_acc[pr];
-#pragma unroll
-              for (int ks = 0; ks < OZ_BK / 32; ++ks) {
-                umma_i8_2cta(tmem_base + acc * 128u, smem_desc_sw64(a_addr + ks * 32), smem_desc_sw64(b_addr + ks * 32),
-                             OZ_IDESC2, (acc_used >> acc) & 1u);
-                acc_used |= 1u << acc;
-              }
-            }
-            umma_commit_2cta(&empty[stage]);
-            if (++stage == OZ2_STAGES) {
-              stage = 0;
-              phase ^= 1;
-            }
-          }
-          umma_commit_2cta(tmem_full);
-        }
-      } else {
-        // ===== relay (peer): my stage is full -> tell the leader =====
-        const uint32_t remote = mapa_shared(smem_u32(peer_full), 0);
-        for (int w = cluster_id; w < nwork; w += nclusters) {
-          const OzWork2 wk = work[w];
-          for (int kb = wk.kb0; kb < wk.kb1; ++kb) {
-            mbar_wait(&full[stage], phase);
-            mbar_arrive_cluster(remote + (uint32_t)stage * 8u);
-            if (++stage == OZ2_STAGES) {
-              stage = 0;
-              phase ^= 1;
-            }
-          }
-        }
-      }
-    }
-  } else {
-    // ===== epilogue (8 warps per CTA; this CTA's 128 rows) =====
-    const int quarter = warp & 3, half = (warp - 2) >> 2;
-    const int row_local = quarter * 32 + lane, col0 = half * 64;
-    const uint32_t tmem_empty_leader = mapa_shared(smem_u32(tmem_empty), 0);
-    int it = 0;
-    for (int w = cluster_id; w < nwork; w += nclusters, ++it) {
-      const OzWork2 wk = work[w];
-      const OzGroup& g = plan.g[wk.group];
-      const int bi = rank ? wk.bi1 : wk.bi0;
-      const bool discard = rank && wk.dup;
-      mbar_wait(tmem_full, (uint32_t)(it & 1));
-      tc_fence_after();
-      double acc[64];
-#pragma unroll
-      for (int j = 0; j < 64; ++j) acc[j] = 0.0;
-      for (int a = 0; a < g.n_acc; ++a) {
-        const double wgt = (double)(1ull << g.acc_shift[a]);
-#pragma unroll
-        for (int c16 = 0; c16 < 4; ++c16) {
-          uint32_t v[16];
-          tmem_ld16(tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(a * 128 + col0 + c16 * 16), v);
-#pragma unroll
-          for (int j = 0; j < 16; ++j) acc[c16 * 16 + j] = fma((double)(int)v[j], wgt, acc[c16 * 16 + j]);
-        }
-      }
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive_cluster(tmem_empty_leader);
-      if (discard) continue;
-      const int r = bi * OZ_BM + row_local;
-      const int er = expo[r];
-      const bool diag = bi == wk.bj;
-      const bool tame = er != OZ_EXPO_BAD && er > -400 && er < 400;
-      const double sr = tame ? __longlong_as_double((long long)(1023 + er + g.exp_base) << 52) : 0.0;
-#pragma unroll
-      for (int j = 0; j < 64; ++j) {
-        const int col = wk.bj * OZ_BM + col0 + j;
-        const int ec = expo[col];
-        double v = acc[j];
-        if (er == OZ_EXPO_BAD || ec == OZ_EXPO_BAD) v = __longlong_as_double(0x7ff8000000000000LL);
-        else if (tame && ec > -400 && ec < 400) v = v * sr * pow2[col];
-        else v = ldexp(v, er + ec + g.exp_base);
-        if (v != 0.0) {
-          // row-major LOWER triangle (csrc/chol.cu factors it; fabric mode: one multimem op per element); the mirror only
-          // for the library factorisation A/B
-          if (!diag || col <= r) {
-            double* q = &Cmat[(size_t)r * Dpad + col];
-            if (mc_off) {
-              asm volatile("multimem.red.relaxed.sys.global.add.f64 [%0], %1;" ::"l"(q + mc_off), "d"(-v) : "memory");
-            } else {
-              atomicAdd(q, -v);
-            }
-          }
-          if (fill_upper && (!diag || col < r)) atomicAdd(&Cmat[(size_t)col * Dpad + r], -v);
-        }
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();                          // nobody leaves while the partner may still address this CTA
-  if (warp == 1) tmem_dealloc2(tmem_base, 512);
-}
-
-
-// ---------------------------------------------------------------------------------------------------------
-// hardware-rule probe (tools/syrk_i8_check.py probe): may a 1-D bulk copy whose destination is the issuing CTA's own
-// shared memory complete on an mbarrier that lives in the OTHER CTA of the cluster?  Measured on B200 (r01): NO -- the
-// bytes land, the remote barrier never completes (out = 0, 1, 1); the barrier has to be in the destination CTA, which
-// is why the CTA-pair SYRK relays "stage full" through a second barrier.  Bounded spin: the probe cannot hang.  out[0] = leader's barrier completed, out[1] = the
-// peer's bytes landed in the peer's buffer, out[2] = the leader's own bytes landed.
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(32, 1)
-    oz_probe_remote_mbar_kernel(const uint8_t* __restrict__ src, int* __restrict__ out) {
-  __shared__ __align__(128) uint8_t buf[256];
-  __shared__ uint64_t bar;
-  const uint32_t rank = cluster_ctarank();
-  const int tid = threadIdx.x;
-  for (int i = tid; i < 256; i += 32) buf[i] = 0;
-  if (tid == 0) {
-    mbar_init(&bar, 1);
-    mbar_fence_init();
-  }
-  fence_proxy_async();
-  __syncthreads();
-  cluster_sync_all();
-  if (tid == 0) {
-    if (rank == 0) {
-      mbar_expect_tx(&bar, 512);
-      tma_load_1d(buf, src, 256, &bar);
-    } else {
-      const uint32_t remote_bar = mapa_shared(smem_u32(&bar), 0);
-      asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                       smem_u32(buf)),
-                   "l"(src + 256), "r"(256), "r"(remote_bar)
-                   : "memory");
-    }
-  }
-  if (rank == 0 && tid == 0) {
-    int done = 0;
-    for (int i = 0; i < 2000000 && !done; ++i) {
-      uint32_t ok;
-      asm volatile(
-          "{\n.reg .pred p;\nmbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}\n"
-          : "=r"(ok)
-          : "r"(smem_u32(&bar)), "r"(0)
-          : "memory");
-      done = (int)ok;
-    }
-    out[0] = done;
-  }
-  // give the copies time either way, then look at the buffers
-  for (int i = 0; i < 200000; ++i) __nanosleep(20);
-  cluster_sync_all();
-  if (tid == 0) {
-    int ok = 1;
-    for (int i = 0; i < 256; ++i) ok &= (buf[i] == src[rank * 256 + i]);
-    out[rank == 0 ? 2 : 1] = ok;
-  }
-  cluster_sync_all();
-}
 
 // ---------------------------------------------------------------------------------------------------------
 // tensor-pipe rate probe (tools/syrk_i8_check.py rate): back-to-back kind::i8 MMAs on resident shared-memory tiles,
@@ -822,16 +432,16 @@ __global__ void __launch_bounds__(128, 1) oz_mma_rate_kernel(int iters, int mode
 
 // ---------------------------------------------------------------------------------------------------------
 // host side: order groups and work list
-bool build_plan(int s, OzPlan* plan, int max_acc) {
+bool build_plan(int s, OzPlan* plan) {
   if (s < 3 || s > 7) return false;
   plan->slices = s;
   const int B = 8 * s - 2;
   const int tlast = s + 1;                       // orders 2 .. s+1 are kept
   int ng = 0;
-  for (int t0 = 2; t0 <= tlast; t0 += max_acc) {
+  for (int t0 = 2; t0 <= tlast; t0 += OZ_MAX_ACC) {
     if (ng >= OZ_MAX_GROUPS) return false;
     OzGroup& g = plan->g[ng++];
-    const int t1 = std::min(t0 + max_acc - 1, tlast);
+    const int t1 = std::min(t0 + OZ_MAX_ACC - 1, tlast);
     g.n_acc = t1 - t0 + 1;
     g.exp_base = 8 * (2 * s - t1) - 2 * B;
     int slot_a[8], slot_b[8];
@@ -869,16 +479,15 @@ bool build_plan(int s, OzPlan* plan, int max_acc) {
 }
 
 
-// Work items are handed out statically (item w goes to CTA / cluster w mod n, longest first), so the finishing time is
+// Work items are handed out statically (item w goes to CTA w mod n, longest first), so the finishing time is
 // the heaviest residue class.  The k-split granularity is chosen by simulating that assignment for a few candidate
 // targets and keeping the best makespan (+ a small charge per item for its epilogue).
 struct OzTileJob {
-  int bi0, bi1, bj, dup;
+  int bi, bj;
   int kb0 = 0, kb1 = -1;       // k-block range in which BOTH row blocks can be non-zero (kb1 < 0: all of K)
 };
-template <class Work, class Make>
-void build_work_list(const OzPlan& plan, const std::vector<OzTileJob>& jobs, int KB, int nworkers, Make make,
-                     std::vector<Work>* out) {
+void build_work_list(const OzPlan& plan, const std::vector<OzTileJob>& jobs, int KB, int nworkers,
+                     std::vector<OzWork>* out) {
   long long total = 0, pairs_all = 0;
   for (int g = 0; g < plan.n_groups; ++g) pairs_all += plan.g[g].n_pairs;
   for (const OzTileJob& jb : jobs) total += pairs_all * (long long)((jb.kb1 < 0 ? KB : jb.kb1) - jb.kb0);
@@ -886,7 +495,7 @@ void build_work_list(const OzPlan& plan, const std::vector<OzTileJob>& jobs, int
   long long best = -1;
   for (int div = 2; div <= 10; ++div) {
     const long long target = std::max<long long>(1, total / ((long long)nworkers * div));
-    std::vector<std::pair<long long, Work>> items;
+    std::vector<std::pair<long long, OzWork>> items;
     for (const OzTileJob& jb : jobs) {
       const int jk0 = jb.kb0, jk1 = jb.kb1 < 0 ? KB : jb.kb1, len = jk1 - jk0;
       if (len <= 0) continue;
@@ -897,7 +506,7 @@ void build_work_list(const OzPlan& plan, const std::vector<OzTileJob>& jobs, int
         parts = std::min(parts, len);
         for (int p = 0; p < parts; ++p) {
           const int k0 = jk0 + (int)((long long)len * p / parts), k1 = jk0 + (int)((long long)len * (p + 1) / parts);
-          items.push_back({(long long)plan.g[g].n_pairs * (k1 - k0), make(jb, g, k0, k1)});
+          items.push_back({(long long)plan.g[g].n_pairs * (k1 - k0), OzWork{jb.bi, jb.bj, g, k0, k1}});
         }
       }
     }
@@ -922,25 +531,8 @@ struct OzHostState {
   std::vector<OzWork> work;
   OzWork* pinned = nullptr;       // page-locked copy of `work`, so the per-call upload is a true async copy
   size_t pinned_cap = 0;
-  std::vector<OzWork2> work2;     // CTA-pair variant
-  OzWork2* pinned2 = nullptr;
-  size_t pinned2_cap = 0;
 };
 
-// VGG_SYRK_TS=1: A operand from tensor memory; default: both operands from shared memory (the r01 kernel)
-bool use_ts_kernel() {
-  static const bool v = [] { const char* e = getenv("VGG_SYRK_TS"); return e && e[0] == '1'; }();
-  return v;
-}
-
-bool use_pair_kernel() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("VGG_SYRK_PAIR");
-    v = (e && e[0] == '1') ? 1 : 0;
-  }
-  return v == 1;
-}
 thread_local OzHostState g_oz;
 
 int oz_max_parts(int KB) { return std::max(16, (KB + OZ_MAX_ITEM_KB - 1) / OZ_MAX_ITEM_KB); }
@@ -952,7 +544,7 @@ size_t oz_workspace_bytes(int Kpad, int Dpad, int s) {
   bytes += align_up((size_t)Dpad * 8, 256);                                   // amax
   bytes += align_up((size_t)Dpad * 4, 256);                                   // expo
   bytes += align_up((size_t)Dpad * 8, 256);                                   // pow2
-  bytes += align_up((size_t)nb * (nb + 1) / 2 * OZ_MAX_GROUPS * oz_max_parts(KB) * sizeof(OzWork2), 256);   // work list (upper bound, either variant)
+  bytes += align_up((size_t)nb * (nb + 1) / 2 * OZ_MAX_GROUPS * oz_max_parts(KB) * sizeof(OzWork), 256);    // work list (upper bound)
   bytes += align_up((size_t)s * nb * KB * OZ_TILE_BYTES, 1024) + 1024;        // slices
   return bytes;
 }
@@ -970,8 +562,7 @@ int syrk_i8_reset_amax(void* ws, int Dpad, cudaStream_t st) {
 }
 
 // Sraw -= Zt^T Zt with s int8 slices.  Zt [Kpad][Dpad] (Dpad % 128 == 0), Cmat [Dpad][Dpad] row-major, LOWER triangle
-// written (plus the mirror when g_fill_upper), same contract as launch_syrk.
-extern int g_fill_upper;      // csrc/ba_schur.cu
+// written.
 // Band hint of the current solve (csrc/ba_solve.cu): [lo, hi) k-block range per 128-column row block of Zt outside which
 // the block is exactly zero; empty = dense.  Tiles whose two ranges do not intersect are skipped, the others shortened.
 std::vector<int> g_syrk_kb_ranges;
@@ -996,18 +587,17 @@ int launch_syrk_i8(int Kpad, int Dpad, const double* Zt, double* Cmat, ptrdiff_t
       VGG_CUDA_CHECK(cudaMemcpyAsync(hs.ranges_dev, hs.ranges.data(), sizeof(int) * hs.ranges.size(), cudaMemcpyHostToDevice, st));
       VGG_CUDA_CHECK(cudaStreamSynchronize(st));          // the source is pageable host memory; once per (re)plan
     }
-    VGG_REQUIRE(build_plan(s, &hs.plan, use_ts_kernel() ? 3 : 4), "syrk_i8: slices must be in [3,7]");
+    VGG_REQUIRE(build_plan(s, &hs.plan), "syrk_i8: slices must be in [3,7]");
     int dev = 0;
     VGG_CUDA_CHECK(cudaGetDevice(&dev));
     VGG_CUDA_CHECK(cudaDeviceGetAttribute(&hs.sms, cudaDevAttrMultiProcessorCount, dev));
-    VGG_CUDA_CHECK(cudaFuncSetAttribute(oz_syrk_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)OZ_SMEM_BYTES));
-    VGG_CUDA_CHECK(cudaFuncSetAttribute(oz_syrk_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)OZ_SMEM_BYTES));
+    VGG_CUDA_CHECK(cudaFuncSetAttribute(oz_syrk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)OZ_SMEM_BYTES));
     // work items: (tile, group, k range), longest first (build_work_list picks the k-split granularity)
     {
       std::vector<OzTileJob> jobs;
       for (int bi = 0; bi < nb; ++bi)
         for (int bj = 0; bj <= bi; ++bj) {                                    // upper tile (row block bj <= column block bi)
-          OzTileJob jb{bj, bj, bi, 0};
+          OzTileJob jb{bj, bi};
           if (banded) {
             jb.kb0 = std::max(hs.ranges[2 * bi], hs.ranges[2 * bj]);
             jb.kb1 = std::min(hs.ranges[2 * bi + 1], hs.ranges[2 * bj + 1]);
@@ -1015,8 +605,7 @@ int launch_syrk_i8(int Kpad, int Dpad, const double* Zt, double* Cmat, ptrdiff_t
           }
           jobs.push_back(jb);
         }
-      build_work_list<OzWork>(hs.plan, jobs, KB, hs.sms,
-                              [](const OzTileJob& j, int g, int k0, int k1) { return OzWork{j.bi0, j.bj, g, k0, k1}; }, &hs.work);
+      build_work_list(hs.plan, jobs, KB, hs.sms, &hs.work);
     }
     if (hs.work.size() > hs.pinned_cap) {
       if (hs.pinned) cudaFreeHost(hs.pinned);
@@ -1024,26 +613,6 @@ int launch_syrk_i8(int Kpad, int Dpad, const double* Zt, double* Cmat, ptrdiff_t
       VGG_CUDA_CHECK(cudaHostAlloc(reinterpret_cast<void**>(&hs.pinned), sizeof(OzWork) * hs.pinned_cap, cudaHostAllocDefault));
     }
     std::copy(hs.work.begin(), hs.work.end(), hs.pinned);
-    // CTA-pair variant: row blocks of one column paired two by two (an odd one out is paired with itself, second half discarded)
-    {
-      VGG_CUDA_CHECK(cudaFuncSetAttribute(oz_syrk_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)OZ2_SMEM_BYTES));
-      const int nclusters = std::max(1, hs.sms / 2);
-      std::vector<OzTileJob> jobs;
-      for (int bj = 0; bj < nb; ++bj)
-        for (int bi = bj; bi < nb; bi += 2) {
-          const bool dup = bi + 1 >= nb;
-          jobs.push_back({bi, dup ? bi : bi + 1, bj, dup ? 1 : 0});
-        }
-      build_work_list<OzWork2>(hs.plan, jobs, KB, nclusters,
-                               [](const OzTileJob& j, int g, int k0, int k1) { return OzWork2{j.bi0, j.bi1, j.bj, g, k0, k1, j.dup}; },
-                               &hs.work2);
-      if (hs.work2.size() > hs.pinned2_cap) {
-        if (hs.pinned2) cudaFreeHost(hs.pinned2);
-        hs.pinned2_cap = hs.work2.size();
-        VGG_CUDA_CHECK(cudaHostAlloc(reinterpret_cast<void**>(&hs.pinned2), sizeof(OzWork2) * hs.pinned2_cap, cudaHostAllocDefault));
-      }
-      std::copy(hs.work2.begin(), hs.work2.end(), hs.pinned2);
-    }
     hs.Kpad = Kpad;
     hs.Dpad = Dpad;
     hs.slices = s;
@@ -1052,16 +621,12 @@ int launch_syrk_i8(int Kpad, int Dpad, const double* Zt, double* Cmat, ptrdiff_t
   unsigned long long* amax = c.take<unsigned long long>(Dpad);
   int* expo = c.take<int>(Dpad);
   double* pow2 = c.take<double>(Dpad);
-  OzWork2* work_raw = c.take<OzWork2>((size_t)nb * (nb + 1) / 2 * OZ_MAX_GROUPS * oz_max_parts(KB));
-  OzWork* work_d = reinterpret_cast<OzWork*>(work_raw);
+  OzWork* work_d = c.take<OzWork>((size_t)nb * (nb + 1) / 2 * OZ_MAX_GROUPS * oz_max_parts(KB));
   c.off = align_up(c.off, 1024);
   int8_t* slices = reinterpret_cast<int8_t*>(c.base + c.off);
   const size_t slice_stride = (size_t)nb * KB * OZ_TILE_BYTES;
   const int nwork = (int)hs.work.size();
-
-  const bool pair = use_pair_kernel() && hs.sms >= 2 && g_fabric_dev.world <= 1 && !banded;   // the reduce-scatter epilogue lives in oz_syrk_kernel
-  if (pair) VGG_CUDA_CHECK(cudaMemcpyAsync(work_raw, hs.pinned2, sizeof(OzWork2) * hs.work2.size(), cudaMemcpyHostToDevice, st));
-  else VGG_CUDA_CHECK(cudaMemcpyAsync(work_d, hs.pinned, sizeof(OzWork) * nwork, cudaMemcpyHostToDevice, st));
+  VGG_CUDA_CHECK(cudaMemcpyAsync(work_d, hs.pinned, sizeof(OzWork) * nwork, cudaMemcpyHostToDevice, st));
   if (!amax_ready) {
     VGG_CUDA_CHECK(cudaMemsetAsync(amax, 0, sizeof(unsigned long long) * Dpad, st));
     const int ksplit = 64;
@@ -1072,20 +637,9 @@ int launch_syrk_i8(int Kpad, int Dpad, const double* Zt, double* Cmat, ptrdiff_t
   oz_slice_kernel<<<dim3(nb, KB), 512, 0, st>>>(Kpad, Dpad, KB, s, Zt, amax, expo, pow2, slices, slice_stride,
                                                 banded ? hs.ranges_dev : nullptr);
   VGG_LAUNCH_CHECK();
-  if (pair) {
-    const int nwork2 = (int)hs.work2.size();
-    const int nclusters = std::min(std::max(1, hs.sms / 2), nwork2);
-    oz_syrk_pair_kernel<<<2 * nclusters, OZ_THREADS, OZ2_SMEM_BYTES, st>>>(hs.plan, work_raw, nwork2, KB, slices, slice_stride,
-                                                                         expo, pow2, Dpad, Cmat, mc_off, g_fill_upper);
-  } else {
-    const int grid = std::min(hs.sms, nwork);
-    if (use_ts_kernel())
-      oz_syrk_kernel<true><<<grid, OZ_THREADS_TS, OZ_SMEM_BYTES, st>>>(hs.plan, work_d, nwork, KB, slices, slice_stride, expo,
-                                                                    pow2, Dpad, Cmat, mc_off, g_fill_upper, g_fabric_dev);
-    else
-      oz_syrk_kernel<false><<<grid, OZ_THREADS, OZ_SMEM_BYTES, st>>>(hs.plan, work_d, nwork, KB, slices, slice_stride, expo,
-                                                                  pow2, Dpad, Cmat, mc_off, g_fill_upper, g_fabric_dev);
-  }
+  const int grid = std::min(hs.sms, nwork);
+  oz_syrk_kernel<<<grid, OZ_THREADS, OZ_SMEM_BYTES, st>>>(hs.plan, work_d, nwork, KB, slices, slice_stride, expo, pow2, Dpad,
+                                                          Cmat, mc_off, g_fabric_dev);
   VGG_LAUNCH_CHECK();
   return VGG_OK;
 }
@@ -1123,28 +677,6 @@ int vgg_syrk_ozaki_mma_rate(int iters, int mode, double* out_cycles, void* strea
   VGG_CUDA_CHECK(cudaMemcpy(&h, d, sizeof(h), cudaMemcpyDeviceToHost));
   cudaFree(d);
   *out_cycles = (double)h / iters;
-  return VGG_OK;
-}
-
-/* Hardware-rule probe for the CTA-pair kernel: out_host[0..2] = (leader barrier completed by a peer-issued bulk copy,
- * peer bytes landed, leader bytes landed).  Bounded spin, cannot hang. */
-int vgg_probe_remote_mbarrier(int* out_host, void* stream) {
-  using namespace vgg;
-  g_launch_count = 0;
-  VGG_REQUIRE(out_host, "null pointer");
-  uint8_t* src = nullptr;
-  int* out = nullptr;
-  VGG_CUDA_CHECK(cudaMalloc(&src, 512));
-  VGG_CUDA_CHECK(cudaMalloc(&out, 16));
-  uint8_t h[512];
-  for (int i = 0; i < 512; ++i) h[i] = (uint8_t)(i * 7 + 3);
-  VGG_CUDA_CHECK(cudaMemcpy(src, h, 512, cudaMemcpyHostToDevice));
-  VGG_CUDA_CHECK(cudaMemset(out, 0xFF, 16));
-  oz_probe_remote_mbar_kernel<<<2, 32, 0, static_cast<cudaStream_t>(stream)>>>(src, out);
-  VGG_LAUNCH_CHECK();
-  VGG_CUDA_CHECK(cudaMemcpy(out_host, out, 12, cudaMemcpyDeviceToHost));
-  cudaFree(src);
-  cudaFree(out);
   return VGG_OK;
 }
 

@@ -23,7 +23,7 @@ constexpr unsigned long long TS_SENTINEL = 0xffffffffffffffffull;   // x is pre-
 
 __global__ void __launch_bounds__(TS_THREADS, 1)
     trsv_upper_kernel(int n, int lda, const double* __restrict__ A, const double* __restrict__ y, size_t y_stride,
-                      double* __restrict__ x, int* flags, int epoch, int use_flag) {
+                      double* __restrict__ x, long long* __restrict__ stamps) {
   extern __shared__ __align__(16) double ts_smem[];
   double(*Ud)[TS_NB + 1] = reinterpret_cast<double(*)[TS_NB + 1]>(ts_smem);                            // diagonal block
   double(*Vi)[TS_NB + 1] = reinterpret_cast<double(*)[TS_NB + 1]>(ts_smem + TS_NB * (TS_NB + 1));      // its inverse
@@ -35,15 +35,14 @@ __global__ void __launch_bounds__(TS_THREADS, 1)
   const int rows = min(TS_NB, n - r0);
   const int tid = threadIdx.x;
   const int r = tid >> 2, seg = tid & 3;      // row of the block, 16-column segment
-  // use_flag == 2 (tools/microbench.py trsv): globaltimer stamps into flags (as int64, 5 per block row): kernel entry,
-  // diagonal block loaded, inverse ready, every x_j consumed, x_b published
-  long long* stamps = reinterpret_cast<long long*>(flags);
+  // stamps (vgg_dev_trsv_probe only, null in the solve): globaltimer stamps, 6 slots per block row: kernel entry,
+  // diagonal block loaded, inverse ready, every x_j consumed, x_b published, right-hand side in place
   auto now_ns = []() {
     long long t;
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
     return t;
   };
-  if (use_flag == 2 && tid == 0) stamps[6 * b] = now_ns();
+  if (stamps && tid == 0) stamps[6 * b] = now_ns();
   // this block row's right-hand side, requested FIRST: r02 timestamps showed this one 8-byte load per thread taking
   // ~19 us when it was issued after the inversion (every block row, same absolute completion time) -- and the whole
   // chain waits for the last block row.  Issued here it completes under the block load and the inversion.
@@ -58,7 +57,7 @@ __global__ void __launch_bounds__(TS_THREADS, 1)
     Ud[i][j] = v;
   }
   __syncthreads();
-  if (use_flag == 2 && tid == 0) stamps[6 * b + 1] = now_ns();
+  if (stamps && tid == 0) stamps[6 * b + 1] = now_ns();
   if (tid < TS_NB) xs[tid] = 1.0 / Ud[tid][tid];       // reciprocal pivots (xs is free until the first hop)
   __syncthreads();
   {
@@ -79,11 +78,11 @@ __global__ void __launch_bounds__(TS_THREADS, 1)
     }
   }
   __syncthreads();
-  if (use_flag == 2 && tid == 0) stamps[6 * b + 2] = now_ns();
+  if (stamps && tid == 0) stamps[6 * b + 2] = now_ns();
   // ---- right-hand side rows of this block
   if (tid < TS_NB) accs[tid] = y_mine;
   __syncthreads();
-  if (use_flag == 2 && tid == 0) stamps[6 * b + 5] = now_ns();
+  if (stamps && tid == 0) stamps[6 * b + 5] = now_ns();
 
   // ---- block columns to the right, last first; tile j+... prefetched into registers before its x is awaited
   // three tiles are kept in flight in registers (tiles do not depend on x, only x_j does)
@@ -98,21 +97,9 @@ __global__ void __launch_bounds__(TS_THREADS, 1)
   auto hop = [&](const double (&tile)[16], int j) {
     // x_j arrives as data: the buffer was pre-filled with a sentinel NaN pattern, every element is polled by one thread
     // (8-byte stores are single-copy atomic, so no flag, no fence and no second round trip are needed)
-    if (use_flag == 1) {
-      // ONE thread of the CTA watches block j's flag (with a short back-off), then 64 threads fetch the block through L2.
-      // The data-as-flag variant below has every waiting CTA poll 64 elements: up to 37 CTAs x 64 threads hammer the
-      // four L2 lines of the newest block, and the producer's stores queue behind them.
-      if (tid == 0) {
-        int seen;
-        while (true) {
-          asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(seen) : "l"(flags + j) : "memory");
-          if (seen == epoch) break;
-          __nanosleep(40);
-        }
-      }
-      __syncthreads();
-      if (tid < TS_NB) xs[tid] = (j * TS_NB + tid < n) ? __ldcg(&x[j * TS_NB + tid]) : 0.0;
-    } else if (tid < TS_NB) {
+    // (r02: one flag per block row watched by one thread per CTA measured 160.6 us against 150.6 us for this hand-off --
+    // the fence + flag round trip costs more than the 64-thread polling it removes)
+    if (tid < TS_NB) {
       double v = 0.0;
       if (j * TS_NB + tid < n) {
         const volatile unsigned long long* src = reinterpret_cast<const volatile unsigned long long*>(&x[j * TS_NB + tid]);
@@ -158,7 +145,7 @@ __global__ void __launch_bounds__(TS_THREADS, 1)
     --j;
   }
   }
-  if (use_flag == 2 && tid == 0) stamps[6 * b + 3] = now_ns();      // every x_j this block row needs has been consumed
+  if (stamps && tid == 0) stamps[6 * b + 3] = now_ns();      // every x_j this block row needs has been consumed
   // reduce the four segments of a row, subtract from the right-hand side
   acc += __shfl_xor_sync(0xffffffffu, acc, 1);
   acc += __shfl_xor_sync(0xffffffffu, acc, 2);
@@ -184,28 +171,16 @@ __global__ void __launch_bounds__(TS_THREADS, 1)
       *reinterpret_cast<volatile unsigned long long*>(&x[r0 + r]) = bits;
     }
   }
-  if (use_flag == 2) {
+  if (stamps) {
     __syncthreads();
     if (tid == 0) stamps[6 * b + 4] = now_ns();
-    return;
-  }
-  if (use_flag) {
-    __syncthreads();                                    // all 64 stores issued
-    if (tid == 0) {
-      __threadfence();
-      asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(flags + b), "r"(epoch) : "memory");
-    }
   }
 }
 
 }  // namespace
 
-size_t trsv_workspace_ints(int n) { return (size_t)((n + TS_NB - 1) / TS_NB) + 1; }
-
-// x = U^-1 y; flags: workspace of trsv_workspace_ints(n) ints that must be zero before the first call and is
-// otherwise left to this function (the last int counts calls so that no reset is needed between them).
-int launch_trsv_upper(int n, int lda, const double* A, const double* y, size_t y_stride, double* x, int* flags,
-                      int epoch, cudaStream_t st) {
+// x = U^-1 y
+int launch_trsv_upper(int n, int lda, const double* A, const double* y, size_t y_stride, double* x, cudaStream_t st) {
   const int nb = (n + TS_NB - 1) / TS_NB;
   VGG_REQUIRE(nb <= 120, "trsv_upper: n too large for one co-resident wave");
   const size_t smem = sizeof(double) * (2 * TS_NB * (TS_NB + 1) + 2 * TS_NB);
@@ -214,18 +189,8 @@ int launch_trsv_upper(int n, int lda, const double* A, const double* y, size_t y
     VGG_CUDA_CHECK(cudaFuncSetAttribute(trsv_upper_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr = true;
   }
-  // VGG_TRSV_POLL=flag: one flag per block row and one polling thread per CTA instead of polling the solution elements
-  // themselves.  Measured r02: 160.6 us against 150.6 us for the data hand-off -- the fence + flag round trip costs more
-  // than the 64-thread polling it removes, so the default stays the data hand-off.
-  static const bool use_flag = [] { const char* e = getenv("VGG_TRSV_POLL"); return e && e[0] == 'f'; }();
-  if (use_flag) {
-    VGG_REQUIRE(flags, "trsv_upper: flag workspace missing");
-    epoch = 1;
-    VGG_CUDA_CHECK(cudaMemsetAsync(flags, 0, sizeof(int) * (size_t)nb, st));    // nobody has published anything yet
-  } else {
-    VGG_CUDA_CHECK(cudaMemsetAsync(x, 0xFF, sizeof(double) * (size_t)n, st));   // sentinel fill: x_j is polled as data
-  }
-  trsv_upper_kernel<<<nb, TS_THREADS, smem, st>>>(n, lda, A, y, y_stride, x, flags, epoch, use_flag ? 1 : 0);
+  VGG_CUDA_CHECK(cudaMemsetAsync(x, 0xFF, sizeof(double) * (size_t)n, st));   // sentinel fill: x_j is polled as data
+  trsv_upper_kernel<<<nb, TS_THREADS, smem, st>>>(n, lda, A, y, y_stride, x, nullptr);
   VGG_LAUNCH_CHECK();
   return VGG_OK;
 }
@@ -248,7 +213,7 @@ extern "C" int vgg_dev_trsv_probe(int n, int lda, const double* A_dev, const dou
   const size_t smem = sizeof(double) * (2 * TS_NB * (TS_NB + 1) + 2 * TS_NB);
   VGG_CUDA_CHECK(cudaFuncSetAttribute(trsv_upper_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   VGG_CUDA_CHECK(cudaMemset(x_dev, 0xFF, sizeof(double) * (size_t)n));
-  trsv_upper_kernel<<<nb, TS_THREADS, smem>>>(n, lda, A_dev, y_dev, 1, x_dev, reinterpret_cast<int*>(d), 1, 2);
+  trsv_upper_kernel<<<nb, TS_THREADS, smem>>>(n, lda, A_dev, y_dev, 1, x_dev, d);
   VGG_LAUNCH_CHECK();
   VGG_CUDA_CHECK(cudaDeviceSynchronize());
   VGG_CUDA_CHECK(cudaMemcpy(stamps_host, d, sizeof(long long) * 6 * nb, cudaMemcpyDeviceToHost));
